@@ -2,6 +2,7 @@
 """bench.py -- FastViTHD images/sec @1024 px + FastVLM TTFT (BASELINE.json metric), one JSON line on stdout.
 
     python bench.py --gpus N --steps K --warmup W            # B200-native arm (this repo)
+    python bench.py ... --dump-outputs DIR                   # also write the last timed step's projected tokens as DIR/projected.npy
     python bench.py --impl reference --gpus N --steps K ...  # CPU arm: the reference algorithm on host cores
     python -m torch.distributed.run --nproc-per-node N ... bench.py --gpus N ...   (N > 1)
 
@@ -44,6 +45,7 @@ METRIC = "fastvithd_images_per_sec_1024px"
 UNIT = "images/s"
 CONFIG4_BATCH = 256     # BASELINE.json configs[3]
 CONFIG4_PASS = 32       # images per library pass (workspace 113 MB per image)
+DUMP_BYTES = 64 * 1024 * 1024     # --dump-outputs writes at most this much (all ranks together)
 FALLBACK_PEAKS = {"hbm_gbs": 6650.0, "bf16_tflops": 1590.0}    # /opt/skills/guides/B200_PROFILING.md fallback
 TC_KERNELS = ("gemm_bf16_tcgen05_kernel", "convffn_tcgen05_kernel", "mlp_cluster_tcgen05_kernel", "mlp_fused_tcgen05_kernel",
               "attention_umma_kernel", "repmixer_umma_kernel")
@@ -197,7 +199,7 @@ def run_reference_arm(args):
     rank = int(os.environ.get("RANK", "0"))
     if rank != 0:
         return 0
-    steps, warmup = max(1, args.steps), max(0, args.warmup)
+    steps, warmup = args.steps, max(0, args.warmup)
     times, cores = cpu_reference_time(steps, warmup)
     ms = 1e3 * sum(times) / len(times)
     val = 1e3 / ms
@@ -286,6 +288,20 @@ def timed_steps(fn, steps, flush, barrier):
         ev[i][1].record()
     barrier()
     return [a.elapsed_time(b) for a, b in ev]
+
+
+def dump_outputs(out_dir, outputs, max_bytes):
+    """Write each [B, ...] output as <out_dir>/<name>.npy in float32.  An output larger than `max_bytes` keeps a fixed, seeded
+    subset of its images, so two builds run with the same arguments can be compared output for output."""
+    import numpy as np
+    import torch
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in outputs.items():
+        keep = max(1, max_bytes // len(outputs) // (t[0].numel() * 4))
+        if t.shape[0] > keep:
+            idx = np.sort(np.random.default_rng(0).choice(t.shape[0], keep, replace=False))
+            t = t.index_select(0, torch.from_numpy(idx).to(t.device))
+        np.save(os.path.join(out_dir, name + ".npy"), t.float().cpu().numpy())
 
 
 def gpu_eager_baseline(dev, batches=(1, 32)):
@@ -406,7 +422,7 @@ def run_gpu_arm(args):
         dist.init_process_group("nccl", device_id=dev)
 
     B = args.batch
-    steps, warmup = max(1, args.steps), max(3, args.warmup)
+    steps, warmup = args.steps, max(3, args.warmup)
     packed = pkg.pack_tower(fx.tower_state_dict())
     packed.update(pkg.pack_projector(fx.projector_state_dict(HIDDEN)))
     eng = pkg.Engine(RES, HIDDEN, 2, B).load(packed, dev)
@@ -433,8 +449,15 @@ def run_gpu_arm(args):
         eng.forward(dev_img, want_tokens=False, want_projected=True)
     barrier()
     sampler = ClockSampler(local_rank).start()
-    step_ms = timed_steps(lambda: eng.forward(dev_img, want_tokens=False, want_projected=True), steps, flush, barrier)
+    last = {}
+
+    def fwd():
+        last["projected"] = eng.forward(dev_img, want_tokens=False, want_projected=True)[1]
+
+    step_ms = timed_steps(fwd, steps, flush, barrier)
     total_ms = sum(step_ms)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"projected" if world == 1 else f"projected_rank{rank}": last["projected"]}, DUMP_BYTES // world)
 
     # ---- end to end through the host-buffer entry (H2D + forward + D2H inside the timed region)
     for _ in range(2):
@@ -633,7 +656,13 @@ def main():
     ap.add_argument("--no-config1", action="store_true", help="reference arm: skip the configs[0] predict.py-flow record")
     ap.add_argument("--sustain-s", type=float, default=2.0)
     ap.add_argument("--quick", action="store_true", help="headline only: no cpu/eager baselines, config4, ttft")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write the projected tokens of the last one as "
+                    "DIR/projected.npy (float32; per rank: projected_rank<r>.npy; at most 64 MB, a seeded subset of images beyond that)")
     args = ap.parse_args()
+    if args.steps is not None and args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the outputs of the b200 arm")
     if args.quick:
         args.no_cpu_baseline = args.no_eager_baseline = args.no_config4 = args.no_ttft = True
         args.sustain_s = 0.0

@@ -9,7 +9,9 @@ What it pins (the reference ships no tests / golden vectors of its own, SURVEY.m
                             tokens [1,16,3072], projected [1,16,896], and for every unit on the
                             path (forward hooks on the reference modules) mean/std/absmax plus
                             256 values at seeded flat indices.
-  * ref_1024_tokens.npy  -- reference tower tokens [1,256,3072] at R=1024 (fp32).
+  * ref_1024_tokens_sample.npz -- fingerprint of the reference tower tokens [1,256,3072] at R=1024
+                            (fp32): shape, mean/std/absmax and 65536 values at seeded flat indices
+                            (the full tensor is 3 MB).
   * ref_b2_256.npz       -- batch-2 tokens at R=256 through the reference's list-input branch
                             (mobileclip_encoder.py:78-83) and tensor branch.
 The oracle restatement must reproduce all of them (tests/test_oracle.py).
@@ -26,18 +28,19 @@ from . import ref_loader
 
 OUT = os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "tests", "golden")
 N_SAMPLES = 256
+N_SAMPLES_1024 = 65536
 PROJ_HIDDEN = 896  # Qwen2-0.5B hidden size
 
 
-def sample_indices(numel, name):
+def sample_indices(numel, name, n=N_SAMPLES):
     seed = int.from_bytes(name.encode()[:8].ljust(8, b"\0"), "little") % (2 ** 31)
     rng = np.random.Generator(np.random.PCG64(seed))
-    return rng.integers(0, numel, size=N_SAMPLES)
+    return rng.integers(0, numel, size=n)
 
 
-def fingerprint(name, t):
+def fingerprint(name, t, n=N_SAMPLES):
     flat = t.detach().float().reshape(-1)
-    idx = sample_indices(flat.numel(), name)
+    idx = sample_indices(flat.numel(), name, n)
     return {
         "shape": np.array(t.shape, dtype=np.int64),
         "stats": np.array([flat.mean().item(), flat.std().item(), flat.abs().max().item()], dtype=np.float64),
@@ -106,7 +109,7 @@ def main():
     tower1024 = ref_loader.reference_tower(1024, sd)
     t1024 = tower1024(fx.synthetic_images(1, 1024))
     assert tuple(t1024.shape) == (1, 256, 3072)
-    np.save(os.path.join(OUT, "ref_1024_tokens.npy"), t1024.numpy())
+    np.savez_compressed(os.path.join(OUT, "ref_1024_tokens_sample.npz"), **fingerprint("tokens_1024", t1024, N_SAMPLES_1024))
     print("R=1024 tokens std %.3f absmax %.2f" % (t1024.std(), t1024.abs().max()))
 
     # ---- fixture sensitivity (SURVEY finding 3): default layer-scale/BN init hides the branches

@@ -9,7 +9,7 @@ import torch
 
 from oracle import fastvithd_oracle as orc
 from oracle import fixture as fx
-from oracle.gen_golden import sample_indices
+from oracle.gen_golden import N_SAMPLES_1024, sample_indices
 
 # fp32 CPU vs fp32 CPU of the same ATen ops; oneDNN may pick other kernels on another host.
 RTOL = 2e-4
@@ -77,10 +77,15 @@ def test_batch2_tensor_and_list_branches(tower_sd, golden_dir):
 
 
 def test_tokens_match_reference_1024(tower_sd, golden_dir):
-    ref = np.load(os.path.join(golden_dir, "ref_1024_tokens.npy"))
+    g = np.load(os.path.join(golden_dir, "ref_1024_tokens_sample.npz"))
     t = orc.tower_forward(fx.synthetic_images(1, 1024), tower_sd)
-    assert tuple(t.shape) == (1, 256, 3072)                     # app/FastVLM/FastVLM.swift:303
-    assert rel_l2(t, ref) < RTOL
+    assert tuple(t.shape) == (1, 256, 3072) == tuple(g["shape"])   # app/FastVLM/FastVLM.swift:303
+    flat = t.reshape(-1)
+    got = flat[torch.from_numpy(sample_indices(flat.numel(), "tokens_1024", N_SAMPLES_1024))]
+    assert rel_l2(got, g["samples"]) < RTOL
+    mean, std, absmax = g["stats"]
+    assert abs(flat.mean().item() - mean) <= RTOL * absmax and abs(flat.std().item() - std) <= RTOL * absmax
+    assert abs(flat.abs().max().item() - absmax) <= RTOL * absmax
 
 
 def test_fixture_is_not_blind(run256, tower_sd, golden_dir):
