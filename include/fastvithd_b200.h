@@ -191,7 +191,8 @@ int fvhd_gemm(fvhd_handle h, void* stream, const void* A, const void* W, const v
               void* D, int M, int N, int K, int act);
 
 /* Test entry: the MHSA core softmax((q 32^-1/2) k^T) v of one attention block (mci.py:675-679) on qkv = [B*N, 3C] bf16 (q | k | v,
- * heads of 32) -> out [B*N, C] bf16; kernel per FVHD_ATTN (u: tcgen05/TMEM, attention_umma.cuh; default: mma.sync). */
+ * heads of 32) -> out [B*N, C] bf16; kernel per FVHD_ATTN as read by fvhd_create for this handle (u: tcgen05/TMEM, attention_umma.cuh;
+ * default: mma.sync). */
 int fvhd_attention(fvhd_handle h, void* stream, const void* qkv, void* out, int batch, int N, int C);
 
 /* Test entry: the second-generation fused ConvFFN kernel (convffn.cuh; one CTA per 128-row tile, packed-half GELU, f16 hidden),
@@ -200,7 +201,8 @@ int fvhd_attention(fvhd_handle h, void* stream, const void* qkv, void* out, int 
 int fvhd_convffn_half(fvhd_handle h, void* stream, const void* z, const void* w1, const void* b1, const void* w2, int w2_is_f16, const void* b2,
                   const void* resid, void* out, int M, int C);
 
-/* Test entry: the RepMixer depthwise pair of one block on the tcgen05 mixer kernel (mixer_umma.cuh), mci.py:808-811 + :921:
+/* Test entry: the RepMixer depthwise pair of one block, mci.py:808-811 + :921, on the kernel FVHD_MIXER selected for this handle at
+ * fvhd_create (default: Toeplitz tcgen05, mixer_tz.cuh):
  *   y = dw3x3(x) + b3,  z = dw7x7(y) + b7;  x, y, z device bf16 NHWC [B,H,W,C]; w3 [9][C], w7 [49][C], b3, b7 [C] fp32 (tap-major,
  *   BN folded).  C % 16 == 0. */
 int fvhd_mixer(fvhd_handle h, void* stream, const void* x, const void* w3, const void* b3, const void* w7, const void* b7,

@@ -75,6 +75,72 @@ typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t,
                                   const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave, CUtensorMapSwizzle,
                                   CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
 
+// Kernel-selection switches.  read_options() reads them from the environment once per handle, in fvhd_create: a switch set
+// after a handle exists does not affect that handle.  Defaults are the measured choices; the other values keep the alternatives
+// selectable for A/B measurements and as references for the tests.
+//
+//   switch               values (default first)    selects
+//   FVHD_NO_GRAPH        unset | 1                 1: forwards launch their steps one by one instead of replaying a captured CUDA graph
+//   FVHD_NO_PDL          unset | 1                 1: plain stream order for every launch (no programmatic dependent launch)
+//   FVHD_NO_SPLITK       unset | 1                 1: small-M GEMMs run one CTA per output tile (no k-slices)
+//   FVHD_GEMM_CS         1 | 2 | 4                 GEMM cluster-size cap.  1: at batch 1 the delivered-bytes rate is the limit and multicast only
+//                                                  reduces L2 reads -- measured no gain (profiles/r01_f_summary.md)
+//   FVHD_NO_FUSED_MLP    unset | 1                 1: every ConvFFN as two GEMMs (reference path of the bit-exactness test); implies the next
+//   FVHD_NO_CLUSTER_MLP  unset | 1                 1: the stage-2 (C = 384) ConvFFN never on the 4-CTA-cluster kernel (mlp_cluster.cuh)
+//   FVHD_CONVFFN         2 | 1                     RepMixer ConvFFN.  2: convffn.cuh, except stage 2 at small batches (cluster kernel);
+//                                                  1: mlp_fused.cuh (C <= 192), cluster kernel or two GEMMs (C = 384)
+//   FVHD_CONVFFN_CS      1 | 2                     2: convffn.cuh as 2-CTA clusters sharing the weight stream by TMA multicast.  Bit-identical, but
+//                                                  measured NEUTRAL at batch 32 (C = 384: 303.5 vs 304.0 us, C = 192: 383.7 vs 386.4 us per launch):
+//                                                  the kernel is bound by its MMA1 -> GELU -> MMA2 chain, not by operand ingest
+//   FVHD_MIXER           unset | z | t | 2 | u | f RepMixer depthwise pair.  unset: Toeplitz products on tcgen05 (mixer_tz.cuh) where a launch has
+//                                                  at least one 64 x 32 x 8 item per SM, mixer_tc.cuh below that; z: Toeplitz everywhere; t: 7x7 on
+//                                                  mma.sync (mixer_tc.cuh, the round-1 / early round-2 default); 2: both convs on mma.sync, 16 ch per
+//                                                  CTA (mixer_tc2.cuh); u: tcgen05 diagonal taps (mixer_umma.cuh: correct, but smem-A-read bound --
+//                                                  602 vs 434 us/img at batch 32, profiles/r02_*); f: FMA pipes (dwconv.cuh).
+//                                                  fvhd_mixer: 2 -> tc2, t -> tc, unset or z -> tz, any other value -> umma
+//   FVHD_MIX_TILE        unset | a | 8 | 1 | 5     set: the FMA-pipe kernels of dwconv.cuh, ahead of FVHD_MIXER.  a: automatic tile (8 x 16 below two
+//                                                  CTAs per SM); 8: 8 x 16 / 128 thr; 1: 16 x 16 / 256 thr; 5: 16 x 16 / 512 thr; other values: as t
+//                                                  (as f under FVHD_MIXER=f)
+//   FVHD_TZ_PAIR         2 | 1..8                  Toeplitz mixer sibling-cluster size (1: plain launch), halved until it divides the channel groups
+//   FVHD_TZ_PDL          3 | 0..3                  Toeplitz mixer: bit 0 = launch with the PDL attribute, bit 1 = trigger the successor early
+//   FVHD_TZ_SKIP         0 | 1..15                 Toeplitz mixer timing experiments: work the kernel skips (MixZParams::dbg)
+//   FVHD_ATTN            a | u | m                 MHSA core.  a: tcgen05 / TMEM (attention_umma.cuh) from 512 tokens, mma.sync below; u / m force
+//                                                  one.  fvhd_attention: u -> tcgen05, any other value -> mma.sync
+//   FVHD_STEM            2 | 1                     2: stem2.cuh (persistent, packed-half GELUs, 16-B patch loads); 1: first-generation stem_kernel
+//   FVHD_LLM_ATTN        unset | f                 LLM prefill attention.  unset: causal_attn_mma_kernel; f: FMA pipes (first version)
+//   FVHD_DEBUG_PLAN      unset | any               set: every GEMM configuration is printed to stderr as a plan is built
+struct Options {
+    bool graph = true, pdl = true, splitk = true, fused_mlp = true, cluster_mlp = true, llm_attn_fma = false, debug_plan = false;
+    int gemm_max_cs = 1, convffn_gen = 2, convffn_cs = 1, stem_gen = 2, tz_pair = 2, tz_pdl = 3, tz_skip = 0;
+    char attn = 'a';
+    char mixer = 0;             // 0: unset (automatic choice per launch); an empty value reads as 'z'
+    char mix_tile = 0;          // 0: unset; an empty value reads as '?' (set, no tile letter)
+};
+
+Options read_options() {
+    Options o;
+    auto one = [](const char* name) { const char* e = getenv(name); return e && e[0] == '1'; };
+    o.graph = !one("FVHD_NO_GRAPH");
+    o.pdl = !one("FVHD_NO_PDL");
+    o.splitk = !one("FVHD_NO_SPLITK");
+    o.fused_mlp = !one("FVHD_NO_FUSED_MLP");
+    o.cluster_mlp = o.fused_mlp && !one("FVHD_NO_CLUSTER_MLP");
+    const char* e;
+    if ((e = getenv("FVHD_GEMM_CS")) && (e[0] == '1' || e[0] == '2' || e[0] == '4')) o.gemm_max_cs = e[0] - '0';
+    if ((e = getenv("FVHD_CONVFFN")) && (e[0] == '1' || e[0] == '2')) o.convffn_gen = e[0] - '0';
+    if ((e = getenv("FVHD_CONVFFN_CS")) && (e[0] == '1' || e[0] == '2')) o.convffn_cs = e[0] - '0';
+    if ((e = getenv("FVHD_MIXER"))) o.mixer = e[0] ? e[0] : 'z';
+    if ((e = getenv("FVHD_MIX_TILE"))) o.mix_tile = e[0] ? e[0] : '?';
+    if ((e = getenv("FVHD_TZ_PAIR")) && e[0] >= '0' && e[0] <= '8') o.tz_pair = e[0] > '0' ? e[0] - '0' : 1;
+    if ((e = getenv("FVHD_TZ_PDL"))) o.tz_pdl = atoi(e);
+    if ((e = getenv("FVHD_TZ_SKIP"))) o.tz_skip = atoi(e);
+    if ((e = getenv("FVHD_ATTN")) && e[0]) o.attn = e[0];
+    o.stem_gen = one("FVHD_STEM") ? 1 : 2;
+    o.llm_attn_fma = (e = getenv("FVHD_LLM_ATTN")) && e[0] == 'f';
+    o.debug_plan = getenv("FVHD_DEBUG_PLAN") != nullptr;
+    return o;
+}
+
 }  // namespace
 
 // LLM prefill engine attached to a handle (row f3): caller-owned weights, library-owned activations / KV cache, one plan per length.
@@ -93,6 +159,7 @@ struct LlmState {
 struct fvhd_handle_s {
     LlmState* llm = nullptr;
     fvhd_config cfg;
+    Options opt;
     std::string err;
     int R = 0, ntok = 0;
     std::vector<WeightSpec> specs;
@@ -107,7 +174,6 @@ struct fvhd_handle_s {
     int cf_clusters[3] = {0, 0, 0};   // resident 2-CTA clusters of convffn_tcgen05_kernel<C, 2>, C = 96 / 192 / 384
     int tz_clusters[9] = {0, 0, 0, 0, 0, 0, 0, 0, 0};   // [cs]: resident cs-CTA clusters of repmixer_tz_kernel (cs = 2, 4, 8)
     int mlpc_clusters = 0;        // resident 4-CTA clusters of mlp_cluster_tcgen05_kernel (cudaOccupancyMaxActiveClusters)
-    bool use_graph = true;
     cudaStream_t cap_stream = nullptr;   // private stream used only to capture graphs (the legacy default stream cannot be captured)
     std::map<int, Plan> plans;
     int64_t act0 = 0;           // elements of the largest activation per image: (R/4)^2 * 96
@@ -288,28 +354,16 @@ Buffers carve(fvhd_handle h, int batch) {
 }
 
 // ------------------------------------------------------------------ launches
-// All kernels go through cudaLaunchKernelEx with programmatic stream serialization (PDL): a kernel may begin its
-// prologue while the previous one drains; the kernels themselves order their global accesses with pdl_wait().
-bool g_use_splitk = true;      // FVHD_NO_SPLITK=1: small-M GEMMs run one CTA per output tile (no k-slices)
+// All kernels go through cudaLaunchKernelEx, with programmatic stream serialization (PDL) unless FVHD_NO_PDL: a kernel may begin
+// its prologue while the previous one drains; the kernels themselves order their global accesses with pdl_wait().
 const size_t kSplitKWsBytes = 32u << 20;
 const int kSplitKTiles = 4096;
-bool g_use_pdl = true;
-int g_gemm_max_cs = 1;        // FVHD_GEMM_CS=1|2|4 caps the GEMM cluster size.  Default 1: at batch 1 the delivered-bytes rate is
-                              // the limit and multicast only reduces L2 reads -- measured no gain (profiles/r01_f_summary.md)
-bool g_use_cluster_mlp = true; // FVHD_NO_CLUSTER_MLP=1: stage-2 (C = 384) ConvFFN as two GEMM launches instead of the 4-CTA-cluster kernel
-bool g_use_fused_mlp = true;  // FVHD_NO_FUSED_MLP=1: ConvFFN as two GEMM launches (reference path of the bit-exactness test)
-const int g_convffn_default = 2;
-const char g_attn_default = 'a';
-char g_attn_mode = 'a';        // FVHD_ATTN=a (default): tcgen05 / TMEM core (attention_umma.cuh) from 512 tokens, mma.sync below; u / m force one
-int g_convffn_gen = 1;         // FVHD_CONVFFN=2 (default): second-generation fused ConvFFN kernel (convffn.cuh); 1: mlp_fused (C <= 192) / two GEMMs
-int g_stem_gen = 2;            // FVHD_STEM=2 (default): stem2.cuh (persistent, packed-half GELUs, 16-B patch loads); 1: first-generation stem_kernel
-char g_mixer_mode = 'z';       // FVHD_MIXER=z (default): 7x7 as Toeplitz products on tcgen05 (mixer_tz.cuh); t: mma.sync 7x7 (mixer_tc.cuh, the round-1 / early
-                               // round-2 default); 2: both convs on mma.sync, 16 ch per CTA (mixer_tc2.cuh); u: tcgen05 diagonal-tap mixer (mixer_umma.cuh: correct, but
-                               // smem-A-read bound -- 602 vs 434 us/img at batch 32, profiles/r02_*); f: FMA pipes (dwconv.cuh)
-unsigned long long* g_gemm_trace = nullptr;   // fvhd_debug_gemm_trace: device buffer, 16 stamps per CTA
-int g_force_bn = 0;                            // fvhd_debug_gemm_trace: force the N tile (0 = cost model)
+// Debug-only, process-wide state of fvhd_debug_gemm_trace (the hook takes no handle).
+unsigned long long* g_gemm_trace = nullptr;   // device buffer, 16 stamps per CTA
+int g_force_bn = 0;                            // force the N tile (0 = cost model)
+int g_debug_gemm_cs = 0;                       // cluster-size cap ahead of the handle's FVHD_GEMM_CS (0 = not set)
 template <typename... KArgs, typename... Args>
-cudaError_t launch_kc(int cluster, void (*kernel)(KArgs...), dim3 grid, dim3 block, size_t smem, cudaStream_t st, Args... args) {
+cudaError_t launch_kc(bool pdl, int cluster, void (*kernel)(KArgs...), dim3 grid, dim3 block, size_t smem, cudaStream_t st, Args... args) {
     cudaLaunchConfig_t cfg = {};
     cfg.gridDim = grid;
     cfg.blockDim = block;
@@ -317,9 +371,7 @@ cudaError_t launch_kc(int cluster, void (*kernel)(KArgs...), dim3 grid, dim3 blo
     cfg.stream = st;
     cudaLaunchAttribute at[2];
     int n = 0;
-    const bool no_pdl = cluster <= 0;    // cluster <= 0: plain stream order for this launch (no programmatic early start); |cluster| = cluster size
-    if (cluster < 0) cluster = -cluster;
-    if (g_use_pdl && !no_pdl) {
+    if (pdl) {
         at[n].id = cudaLaunchAttributeProgrammaticStreamSerialization;
         at[n].val.programmaticStreamSerializationAllowed = 1;
         ++n;
@@ -336,13 +388,28 @@ cudaError_t launch_kc(int cluster, void (*kernel)(KArgs...), dim3 grid, dim3 blo
     return cudaLaunchKernelEx(&cfg, kernel, KArgs(args)...);
 }
 template <typename... KArgs, typename... Args>
-cudaError_t launch_k(void (*kernel)(KArgs...), dim3 grid, dim3 block, size_t smem, cudaStream_t st, Args... args) {
-    return launch_kc(1, kernel, grid, block, smem, st, args...);
+cudaError_t launch_k(bool pdl, void (*kernel)(KArgs...), dim3 grid, dim3 block, size_t smem, cudaStream_t st, Args... args) {
+    return launch_kc(pdl, 1, kernel, grid, block, smem, st, args...);
 }
 
 // ------------------------------------------------------------------ CUDA lazy init
 template <typename K> cudaError_t set_smem(K kernel, size_t bytes) {
     return cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes);
+}
+
+// How many cs-CTA clusters of `kernel` can be resident at once (clusters are placed per GPC); 0 when the query fails.
+template <typename K> int resident_clusters(K kernel, int cs, int threads, size_t smem, int num_sms) {
+    cudaLaunchConfig_t cfg = {};
+    cfg.gridDim = dim3((unsigned)(num_sms / cs * cs));
+    cfg.blockDim = dim3(threads);
+    cfg.dynamicSmemBytes = smem;
+    cudaLaunchAttribute at[1];
+    at[0].id = cudaLaunchAttributeClusterDimension;
+    at[0].val.clusterDim.x = (unsigned)cs; at[0].val.clusterDim.y = 1; at[0].val.clusterDim.z = 1;
+    cfg.attrs = at; cfg.numAttrs = 1;
+    int nc = 0;
+    if (cudaOccupancyMaxActiveClusters(&nc, kernel, &cfg) != cudaSuccess) { nc = 0; (void)cudaGetLastError(); }
+    return nc;
 }
 
 int ensure_cuda(fvhd_handle h) {
@@ -357,28 +424,11 @@ int ensure_cuda(fvhd_handle h) {
     CUDA_TRY(h, cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &fn, cudaEnableDefault, &qres));
     if (!fn || qres != cudaDriverEntryPointSuccess) return fail(h, FVHD_ERR_CUDA, "cuTensorMapEncodeTiled not available from the driver");
     h->encode = reinterpret_cast<EncodeTiledFn>(fn);
-    h->num_sms = prop.multiProcessorCount;
-    { const char* e = getenv("FVHD_NO_GRAPH"); h->use_graph = !(e && e[0] == '1'); }
-    { const char* e = getenv("FVHD_NO_PDL"); g_use_pdl = !(e && e[0] == '1'); }
-    { const char* e = getenv("FVHD_NO_FUSED_MLP"); g_use_fused_mlp = !(e && e[0] == '1'); }
-    { const char* e = getenv("FVHD_NO_CLUSTER_MLP"); g_use_cluster_mlp = g_use_fused_mlp && !(e && e[0] == '1'); }
-    { const char* e = getenv("FVHD_GEMM_CS"); if (e && (e[0] == '1' || e[0] == '2' || e[0] == '4')) g_gemm_max_cs = e[0] - '0'; }
+    const int n = h->num_sms = prop.multiProcessorCount;
     CUDA_TRY(h, set_smem(gemm_bf16_tcgen05_kernel, 227 * 1024));
     CUDA_TRY(h, set_smem(mlp_fused_tcgen05_kernel, 227 * 1024));
     CUDA_TRY(h, set_smem(mlp_cluster_tcgen05_kernel, MLPC_SMEM));
-    {   // how many 4-CTA clusters of the stage-2 ConvFFN kernel can be resident at once (GPC granularity)
-        cudaLaunchConfig_t cfg = {};
-        cfg.gridDim = dim3((unsigned)(prop.multiProcessorCount / MLPC_CS * MLPC_CS));
-        cfg.blockDim = dim3(MLPC_THREADS);
-        cfg.dynamicSmemBytes = MLPC_SMEM;
-        cudaLaunchAttribute at[1];
-        at[0].id = cudaLaunchAttributeClusterDimension;
-        at[0].val.clusterDim.x = MLPC_CS; at[0].val.clusterDim.y = 1; at[0].val.clusterDim.z = 1;
-        cfg.attrs = at; cfg.numAttrs = 1;
-        int nc = 0;
-        if (cudaOccupancyMaxActiveClusters(&nc, mlp_cluster_tcgen05_kernel, &cfg) != cudaSuccess) { nc = 0; (void)cudaGetLastError(); }
-        h->mlpc_clusters = nc;
-    }
+    h->mlpc_clusters = resident_clusters(mlp_cluster_tcgen05_kernel, MLPC_CS, MLPC_THREADS, MLPC_SMEM, n);
     CUDA_TRY(h, set_smem(repmixer_dw_kernel<16, 16, 256>, MixCfgT<16, 16>::SMEM));
     CUDA_TRY(h, set_smem(repmixer_dw_kernel<8, 16, 128>, MixCfgT<8, 16>::SMEM));
     CUDA_TRY(h, set_smem(repmixer_dw_kernel<16, 16, 512, 6, 4, 2>, MixCfgT<16, 16>::SMEM));
@@ -386,48 +436,17 @@ int ensure_cuda(fvhd_handle h) {
     CUDA_TRY(h, set_smem(repmixer_umma_kernel, MixU::SMEM));
     CUDA_TRY(h, set_smem(repmixer_tc2_kernel, MixT2::SMEM));
     CUDA_TRY(h, set_smem(repmixer_tz_kernel, MixZ::SMEM));
-    for (int cs = 2; cs <= 8; cs *= 2) {   // how many sibling clusters of the Toeplitz mixer can be resident at once (GPC granularity)
-        cudaLaunchConfig_t cfg = {};
-        cfg.gridDim = dim3((unsigned)(prop.multiProcessorCount / cs * cs));
-        cfg.blockDim = dim3(MixZ::THREADS);
-        cfg.dynamicSmemBytes = MixZ::SMEM;
-        cudaLaunchAttribute at[1];
-        at[0].id = cudaLaunchAttributeClusterDimension;
-        at[0].val.clusterDim.x = (unsigned)cs; at[0].val.clusterDim.y = 1; at[0].val.clusterDim.z = 1;
-        cfg.attrs = at; cfg.numAttrs = 1;
-        int nc = 0;
-        if (cudaOccupancyMaxActiveClusters(&nc, repmixer_tz_kernel, &cfg) != cudaSuccess) { nc = 0; (void)cudaGetLastError(); }
-        h->tz_clusters[cs] = nc;
-    }
-    { const char* e = getenv("FVHD_MIXER"); g_mixer_mode = (e && e[0]) ? e[0] : 'z'; }
-    { const char* e = getenv("FVHD_ATTN"); g_attn_mode = (e && e[0]) ? e[0] : g_attn_default; }
+    for (int cs = 2; cs <= 8; cs *= 2) h->tz_clusters[cs] = resident_clusters(repmixer_tz_kernel, cs, MixZ::THREADS, MixZ::SMEM, n);
     CUDA_TRY(h, set_smem(attention_umma_kernel, AttU::SMEM));
-    { const char* e = getenv("FVHD_CONVFFN"); g_convffn_gen = (e && e[0] == '2') ? 2 : (e && e[0] == '1') ? 1 : g_convffn_default; }
     CUDA_TRY(h, (set_smem(convffn_tcgen05_kernel<96, 1>, CfCfg<96>::SMEM)));
     CUDA_TRY(h, (set_smem(convffn_tcgen05_kernel<192, 1>, CfCfg<192>::SMEM)));
     CUDA_TRY(h, (set_smem(convffn_tcgen05_kernel<384, 1>, CfCfg<384>::SMEM)));
     CUDA_TRY(h, (set_smem(convffn_tcgen05_kernel<96, 2>, CfCfg<96>::SMEM)));
     CUDA_TRY(h, (set_smem(convffn_tcgen05_kernel<192, 2>, CfCfg<192>::SMEM)));
     CUDA_TRY(h, (set_smem(convffn_tcgen05_kernel<384, 2>, CfCfg<384>::SMEM)));
-    {   // resident 2-CTA clusters of the weight-sharing ConvFFN variant, per C
-        const size_t sm[3] = {CfCfg<96>::SMEM, CfCfg<192>::SMEM, CfCfg<384>::SMEM};
-        for (int ci = 0; ci < 3; ++ci) {
-            cudaLaunchConfig_t cfg = {};
-            cfg.gridDim = dim3((unsigned)(prop.multiProcessorCount / 2 * 2));
-            cfg.blockDim = dim3(CF_THREADS);
-            cfg.dynamicSmemBytes = sm[ci];
-            cudaLaunchAttribute at[1];
-            at[0].id = cudaLaunchAttributeClusterDimension;
-            at[0].val.clusterDim.x = 2; at[0].val.clusterDim.y = 1; at[0].val.clusterDim.z = 1;
-            cfg.attrs = at; cfg.numAttrs = 1;
-            int nc = 0;
-            cudaError_t e = ci == 0 ? cudaOccupancyMaxActiveClusters(&nc, convffn_tcgen05_kernel<96, 2>, &cfg)
-                          : ci == 1 ? cudaOccupancyMaxActiveClusters(&nc, convffn_tcgen05_kernel<192, 2>, &cfg)
-                                    : cudaOccupancyMaxActiveClusters(&nc, convffn_tcgen05_kernel<384, 2>, &cfg);
-            if (e != cudaSuccess) { nc = 0; (void)cudaGetLastError(); }
-            h->cf_clusters[ci] = nc;
-        }
-    }
+    h->cf_clusters[0] = resident_clusters(convffn_tcgen05_kernel<96, 2>, 2, CF_THREADS, CfCfg<96>::SMEM, n);
+    h->cf_clusters[1] = resident_clusters(convffn_tcgen05_kernel<192, 2>, 2, CF_THREADS, CfCfg<192>::SMEM, n);
+    h->cf_clusters[2] = resident_clusters(convffn_tcgen05_kernel<384, 2>, 2, CF_THREADS, CfCfg<384>::SMEM, n);
     CUDA_TRY(h, set_smem(dwconv_kernel<7, 1, 1, 0, 16, 16, 8>, DwCfg<7, 1, 1, 16, 16>::SMEM));
     CUDA_TRY(h, set_smem(dwconv_kernel<7, 1, 1, 0, 8, 16, 8>, DwCfg<7, 1, 1, 8, 16>::SMEM));
     CUDA_TRY(h, set_smem(dwconv_kernel<7, 2, 2, 1, 8, 8, 4>, DwCfg<7, 2, 2, 8, 8>::SMEM));
@@ -438,9 +457,7 @@ int ensure_cuda(fvhd_handle h) {
     CUDA_TRY(h, set_smem(stem2_kernel<float>, Stem2::SMEM));
     CUDA_TRY(h, set_smem(stem2_kernel<__half>, Stem2::SMEM));
     CUDA_TRY(h, set_smem(stem2_kernel<bf16>, Stem2::SMEM));
-    { const char* e = getenv("FVHD_STEM"); g_stem_gen = (e && e[0] == '1') ? 1 : 2; }
     CUDA_TRY(h, cudaStreamCreateWithFlags(&h->cap_stream, cudaStreamNonBlocking));
-    { const char* e = getenv("FVHD_NO_SPLITK"); g_use_splitk = !(e && e[0] == '1'); }
     CUDA_TRY(h, cudaMalloc(&h->splitk_ws, kSplitKWsBytes));
     CUDA_TRY(h, cudaMalloc(&h->splitk_cnt, kSplitKTiles * sizeof(int)));
     CUDA_TRY(h, cudaMemset(h->splitk_cnt, 0, kSplitKTiles * sizeof(int)));
@@ -513,8 +530,68 @@ int make_mixer_umma_step(fvhd_handle h, Step* st, const bf16* x, bf16* y, bf16* 
     int rc = make_tmap_chunked(h, &tm, x, batch, H, W, C, MixU::P, MixU::XH);
     if (rc != FVHD_OK) return rc;
     const dim3 grid((unsigned)(per * mp.groups));
+    const bool pdl = h->opt.pdl;
     *st = [=](cudaStream_t s, const RunCtx&) -> cudaError_t {
-        return launch_k(repmixer_umma_kernel, grid, dim3(MixU::THREADS), MixU::SMEM, s, tm, mp);
+        return launch_k(pdl, repmixer_umma_kernel, grid, dim3(MixU::THREADS), MixU::SMEM, s, tm, mp);
+    };
+    return FVHD_OK;
+}
+
+// RepMixer depthwise pair with the 7x7 on mma.sync (mixer_tc.cuh): persistent CTAs, ~two per SM in total, each bound to one
+// 32-channel group and walking that group's (image, 16 x 16 tile) items.
+int make_mixer_tc_step(fvhd_handle h, Step* st, const bf16* x, bf16* y, bf16* z, const float* w3, const float* b3, const float* w7,
+                       const float* b7, int batch, int H, int W, int C) {
+    if (C % DW_CG) return fail(h, FVHD_ERR_INVALID, "mma.sync mixer needs C %% 32 == 0 (got %d)", C);
+    const int tx = (W + 15) / 16, ty = (H + 15) / 16;
+    int per_group = (2 * h->num_sms) / (C / DW_CG);       // floor: a CTA beyond the resident slots would run its whole item loop as a second wave
+    if (per_group < 1) per_group = 1;
+    if (per_group > tx * ty * batch) per_group = tx * ty * batch;
+    const dim3 grid(per_group, C / DW_CG, 1);
+    CUtensorMap tm;
+    int rc = make_tmap_nhwc(h, &tm, x, batch, H, W, C, MixTc::XP, MixTc::XH);
+    if (rc != FVHD_OK) return rc;
+    const bool pdl = h->opt.pdl;
+    *st = [=](cudaStream_t s, const RunCtx&) -> cudaError_t {
+        return launch_k(pdl, repmixer_tc_kernel, grid, dim3(MixTc::NT), MixTc::SMEM, s, tm, y, z, w3, b3, w7, b7, H, W, C, tx, batch);
+    };
+    return FVHD_OK;
+}
+
+// RepMixer depthwise pair with both convs on mma.sync, 16 channels per CTA (mixer_tc2.cuh).
+int make_mixer_tc2_step(fvhd_handle h, Step* st, const bf16* x, bf16* y, bf16* z, const float* w3, const float* b3, const float* w7,
+                        const float* b7, int batch, int H, int W, int C) {
+    if (C % MixT2::CG) return fail(h, FVHD_ERR_INVALID, "mma.sync mixer (16-channel groups) needs C %% 16 == 0 (got %d)", C);
+    const int tx = (W + MixT2::TOW - 1) / MixT2::TOW, ty = (H + MixT2::TOH - 1) / MixT2::TOH;
+    const dim3 grid(tx * ty, C / MixT2::CG, batch);
+    CUtensorMap tm;
+    int rc = make_tmap_nhwc(h, &tm, x, batch, H, W, C, MixT2::XP, MixT2::XH, MixT2::CG);
+    if (rc != FVHD_OK) return rc;
+    const bool pdl = h->opt.pdl;
+    *st = [=](cudaStream_t s, const RunCtx&) -> cudaError_t {
+        return launch_k(pdl, repmixer_tc2_kernel, grid, dim3(MixT2::NT), MixT2::SMEM, s, tm, y, z, w3, b3, w7, b7, H, W, C, tx);
+    };
+    return FVHD_OK;
+}
+
+// RepMixer depthwise pair on the FMA pipes (dwconv.cuh), one CTA per (tile, 32-channel group, image); the tile per FVHD_MIX_TILE.
+int make_mixer_dw_step(fvhd_handle h, Step* st, const bf16* x, bf16* y, bf16* z, const float* w3, const float* b3, const float* w7,
+                       const float* b7, int batch, int H, int W, int C) {
+    if (C % DW_CG) return fail(h, FVHD_ERR_INVALID, "FMA-pipe mixer needs C %% 32 == 0 (got %d)", C);
+    const long ctas16 = (long)((W + 15) / 16) * ((H + 15) / 16) * (C / DW_CG) * batch;
+    const char t = h->opt.mix_tile;
+    const bool small = t == '8' || (t == 'a' && ctas16 < 2L * h->num_sms), wide = t == '5';
+    const int TH = small ? 8 : 16;
+    const int tx = (W + 15) / 16, ty = (H + TH - 1) / TH;
+    const dim3 grid(tx * ty, C / DW_CG, batch);
+    CUtensorMap tm;
+    int rc = make_tmap_nhwc(h, &tm, x, batch, H, W, C, small ? MixCfgT<8, 16>::XP : MixCfgT<16, 16>::XP,
+                            small ? MixCfgT<8, 16>::XH : MixCfgT<16, 16>::XH);
+    if (rc != FVHD_OK) return rc;
+    const bool pdl = h->opt.pdl;
+    *st = [=](cudaStream_t s, const RunCtx&) -> cudaError_t {
+        if (wide) return launch_k(pdl, repmixer_dw_kernel<16, 16, 512, 6, 4, 2>, grid, dim3(512), MixCfgT<16, 16>::SMEM, s, tm, y, z, w3, b3, w7, b7, H, W, C, tx);
+        if (small) return launch_k(pdl, repmixer_dw_kernel<8, 16, 128>, grid, dim3(128), MixCfgT<8, 16>::SMEM, s, tm, y, z, w3, b3, w7, b7, H, W, C, tx);
+        return launch_k(pdl, repmixer_dw_kernel<16, 16, 256>, grid, dim3(256), MixCfgT<16, 16>::SMEM, s, tm, y, z, w3, b3, w7, b7, H, W, C, tx);
     };
     return FVHD_OK;
 }
@@ -531,10 +608,7 @@ int make_mixer_tz_step(fvhd_handle h, Step* st, const bf16* x, bf16* y, bf16* z,
     mp.tiles_y = (H + MixZ::ZR - 1) / MixZ::ZR;
     mp.groups = C / MixZ::CG;
     const int n_sp = batch * mp.tiles_x * mp.tiles_y;
-    // sibling clusters: FVHD_TZ_PAIR = cluster size (default 2; 1 = plain launch); must divide the number of channel groups
-    int cs = 2;
-    { const char* e = getenv("FVHD_TZ_PAIR"); if (e && e[0] >= '0' && e[0] <= '8') cs = e[0] - '0'; }
-    if (cs < 1) cs = 1;
+    int cs = h->opt.tz_pair;                            // sibling clusters: must divide the number of channel groups
     while (cs > 1 && (mp.groups % cs || h->tz_clusters[cs] <= 0)) cs >>= 1;
     mp.pair_sync = cs > 1 ? cs : 0;
     int slots = cs > 1 ? h->tz_clusters[cs] * cs : h->num_sms;      // resident CTAs (one per SM; clusters are placed per GPC)
@@ -543,12 +617,9 @@ int make_mixer_tz_step(fvhd_handle h, Step* st, const bf16* x, bf16* y, bf16* z,
     if (per < 1) per = 1;
     if (per > n_sp) per = n_sp;
     mp.ctas_per_group = per;
-    { const char* e = getenv("FVHD_TZ_SKIP"); mp.dbg = e ? atoi(e) : 0; }
-    int tz_pdl = 3;          // FVHD_TZ_PDL bits: 1 = launch with the programmatic-serialization attribute, 2 = trigger the successor early
-    { const char* e = getenv("FVHD_TZ_PDL"); if (e) tz_pdl = atoi(e); }
-    mp.pdl_trigger = (tz_pdl & 2) ? 1 : 0;
-    const bool attr = (tz_pdl & 1) != 0;
-    const int pair = cs;
+    mp.dbg = h->opt.tz_skip;
+    mp.pdl_trigger = (h->opt.tz_pdl & 2) ? 1 : 0;
+    const bool pdl = h->opt.pdl && (h->opt.tz_pdl & 1);
     CUtensorMap tm;
     int rc = make_tmap_nhwc(h, &tm, x, batch, H, W, C, MixZ::XP, MixZ::XR, MixZ::CG);
     if (rc != FVHD_OK) return rc;
@@ -556,10 +627,32 @@ int make_mixer_tz_step(fvhd_handle h, Step* st, const bf16* x, bf16* y, bf16* z,
     if ((rc = make_tmap_nhwc(h, &tmz, z, batch, H, W, C, 1, MixZ::ZR, MixZ::CG)) != FVHD_OK) return rc;
     const dim3 grid((unsigned)(per * mp.groups));
     *st = [=](cudaStream_t s, const RunCtx&) -> cudaError_t {
-        return launch_kc(pair > 1 ? (attr ? pair : -pair) : (attr ? 1 : 0), repmixer_tz_kernel, grid, dim3(MixZ::THREADS), MixZ::SMEM, s, tm, tmz, mp);
+        return launch_kc(pdl, cs, repmixer_tz_kernel, grid, dim3(MixZ::THREADS), MixZ::SMEM, s, tm, tmz, mp);
     };
     return FVHD_OK;
 }
+
+// The RepMixer depthwise pair's kernels.  choose_mixer() is the plan's choice; fvhd_mixer maps FVHD_MIXER directly.
+enum class Mixer { Tz, Tc, Tc2, Umma, Dw };
+
+Mixer choose_mixer(fvhd_handle h, int batch, int H, int W, int C) {
+    const char m = h->opt.mixer;
+    if (h->opt.mix_tile) return (strchr("a815", h->opt.mix_tile) || m == 'f') ? Mixer::Dw : Mixer::Tc;
+    if (m == '2' && C % MixT2::CG == 0) return Mixer::Tc2;
+    if (m == 'u') return Mixer::Umma;
+    if (m == 0 || m == 'z') {
+        // Toeplitz tcgen05 mixer whenever there is at least one 64 x 32 x 8 item per SM; below that (stage 2 of a single
+        // 1024-px image: 96 items) the finer-grained mma.sync kernel of mixer_tc.cuh has the shorter critical path
+        // (16 vs 20 us per launch at batch 1).  An explicit FVHD_MIXER=z forces it everywhere.
+        const long items = (long)batch * ((W + MixZ::ZC - 1) / MixZ::ZC) * ((H + MixZ::ZR - 1) / MixZ::ZR) * (C / MixZ::CG);
+        if (m == 'z' || items >= h->num_sms || C % DW_CG != 0) return Mixer::Tz;
+    }
+    return m == 'f' ? Mixer::Dw : Mixer::Tc;
+}
+
+const struct { const char* kernel; decltype(&make_mixer_tz_step) make; } kMixers[] = {     // indexed by Mixer
+    {"repmixer_tz_kernel", make_mixer_tz_step}, {"repmixer_tc_kernel", make_mixer_tc_step}, {"repmixer_tc2_kernel", make_mixer_tc2_step},
+    {"repmixer_umma_kernel", make_mixer_umma_step}, {"repmixer_dw_kernel", make_mixer_dw_step}};
 
 // GEMM configuration = (BN, cluster size CS, which operand the cluster shares).  Cost model per CTA tile (cycles):
 //   load = num_kb * bytes_per_kblock / 36 B/clk   (gemm_trace: ~70 GB/s per SM while all SMs pull, ~10 TB/s chip-wide)
@@ -567,7 +660,7 @@ int make_mixer_tz_step(fvhd_handle h, Step* st, const bf16* x, bf16* y, bf16* z,
 //   epi  = 128 * BN * (GELU ? 10 : 6) / 256       (8 epilogue warps)
 //   tile = max(load, mma, epi) + 400 ;  total = rounds * tile, rounds = ceil(cluster_tiles / resident_clusters)
 struct GemmCfg { int bn, cs, share_b; long cost; int split; };
-GemmCfg pick_gemm_cfg(int M, int N, int K, int act, int num_sms, bool allow_split = false) {
+GemmCfg pick_gemm_cfg(int M, int N, int K, int act, int num_sms, int max_cs, bool allow_split) {
     const int tiles_m = (M + GEMM_BM - 1) / GEMM_BM;
     const int num_kb = (K + GEMM_BK - 1) / GEMM_BK;
     const int cands[5] = {256, 128, 96, 64, 32};
@@ -577,7 +670,7 @@ GemmCfg pick_gemm_cfg(int M, int N, int K, int act, int num_sms, bool allow_spli
         if (bn == 256 && N % 256) continue;
         if (bn > 32 && bn > ((N + 31) / 32) * 32) continue;
         const int tiles_n = (N + bn - 1) / bn;
-        for (int cs = 1; cs <= g_gemm_max_cs; cs *= 2) {
+        for (int cs = 1; cs <= max_cs; cs *= 2) {
             for (int share_b = 0; share_b < (cs == 1 ? 1 : 2); ++share_b) {
                 if (cs > 1 && share_b && (bn / cs) % 8) continue;          // slice boxes stay whole swizzle atoms
                 if (cs > 1 && share_b && tiles_m < cs) continue;
@@ -619,8 +712,8 @@ GemmCfg pick_gemm_cfg(int M, int N, int K, int act, int num_sms, bool allow_spli
 int make_gemm_step(fvhd_handle h, Step* out, const IoBlock* io, int rows_per_image, const bf16* A, int lda, const bf16* W, const float* bias, const bf16* residual, int ldr,
                    bf16* D, int ldd, int M, int N, int K, int act) {
     if (N % 8 || K % 8) return fail(h, FVHD_ERR_INVALID, "GEMM N (%d) and K (%d) must be multiples of 8", N, K);
-    const bool can_split = g_use_splitk && D != nullptr && h->splitk_ws && N % 4 == 0 && ldd % 4 == 0 && (residual == nullptr || ldr % 4 == 0);
-    GemmCfg c = pick_gemm_cfg(M, N, K, act, h->num_sms, can_split);
+    const bool can_split = h->opt.splitk && D != nullptr && h->splitk_ws && N % 4 == 0 && ldd % 4 == 0 && (residual == nullptr || ldr % 4 == 0);
+    GemmCfg c = pick_gemm_cfg(M, N, K, act, h->num_sms, g_debug_gemm_cs ? g_debug_gemm_cs : h->opt.gemm_max_cs, can_split);
     if (g_force_bn) { c.bn = g_force_bn; c.cs = 1; c.share_b = 0; c.split = 1; }
     GemmParams p{};
     p.M = M; p.N = N; p.K = K;
@@ -652,29 +745,17 @@ int make_gemm_step(fvhd_handle h, Step* out, const IoBlock* io, int rows_per_ima
         td = ta;
     }
     const size_t smem = gemm_smem_bytes(p.BN, p.stages);
-    int resident = h->num_sms / p.cs;
-    if (p.cs > 1) {     // how many clusters of this shape can be co-resident (GPC granularity)
-        cudaLaunchConfig_t cfg = {};
-        cfg.gridDim = dim3((unsigned)(h->num_sms / p.cs * p.cs));
-        cfg.blockDim = dim3(GEMM_THREADS);
-        cfg.dynamicSmemBytes = smem;
-        cudaLaunchAttribute at[1];
-        at[0].id = cudaLaunchAttributeClusterDimension;
-        at[0].val.clusterDim.x = (unsigned)p.cs; at[0].val.clusterDim.y = 1; at[0].val.clusterDim.z = 1;
-        cfg.attrs = at; cfg.numAttrs = 1;
-        int nc = 0;
-        cudaError_t e = cudaOccupancyMaxActiveClusters(&nc, gemm_bf16_tcgen05_kernel, &cfg);
-        if (e != cudaSuccess || nc < 1) return fail(h, FVHD_ERR_CUDA, "cudaOccupancyMaxActiveClusters(cs=%d): %s (%d)", p.cs, cudaGetErrorString(e), nc);
-        resident = nc;
-    }
+    const int resident = p.cs > 1 ? resident_clusters(gemm_bf16_tcgen05_kernel, p.cs, GEMM_THREADS, smem, h->num_sms) : h->num_sms;
+    if (resident < 1) return fail(h, FVHD_ERR_CUDA, "no resident %d-CTA cluster of the GEMM kernel (%zu B of shared memory)", p.cs, smem);
     const int nclusters = p.ctiles < resident ? p.ctiles : resident;
     const dim3 grid((unsigned)(nclusters * p.cs));
-    if (getenv("FVHD_DEBUG_PLAN"))
+    if (h->opt.debug_plan)
         fprintf(stderr, "[fvhd] gemm M=%d N=%d K=%d BN=%d stages=%d tiles=%dx%d split_k=%d kb/slice=%d items=%d grid=%u tma_store=%d act=%d\n", M, N, K, p.BN, p.stages,
                 p.tiles_m, p.tiles_n, p.split_k, p.kb_per_split, p.ctiles, grid.x, p.tma_store, act);
     const int cs = p.cs;
+    const bool pdl = h->opt.pdl;
     *out = [=](cudaStream_t s, const RunCtx&) -> cudaError_t {
-        return launch_kc(cs, gemm_bf16_tcgen05_kernel, grid, dim3(GEMM_THREADS), smem, s, ta, tb, td, p);
+        return launch_kc(pdl, cs, gemm_bf16_tcgen05_kernel, grid, dim3(GEMM_THREADS), smem, s, ta, tb, td, p);
     };
     return FVHD_OK;
 }
@@ -689,8 +770,9 @@ int make_dw_step(fvhd_handle h, Step* out_step, const bf16* in, bf16* out, const
     CUtensorMap tm;
     int rc = make_tmap_nhwc(h, &tm, in, batch, H, W, C, Cfg::IWP, Cfg::IH);
     if (rc != FVHD_OK) return rc;
+    const bool pdl = h->opt.pdl;
     *out_step = [=](cudaStream_t s, const RunCtx&) -> cudaError_t {
-        return launch_k(dwconv_kernel<KS, S, MULT, ACT, TOH, TOW, SW>, grid, dim3(DW_THREADS), smem, s, tm, out, w, b, H, W, C, Ho, Wo, tx);
+        return launch_k(pdl, dwconv_kernel<KS, S, MULT, ACT, TOH, TOW, SW>, grid, dim3(DW_THREADS), smem, s, tm, out, w, b, H, W, C, Ho, Wo, tx);
     };
     return FVHD_OK;
 }
@@ -739,16 +821,10 @@ int make_fused_mlp_step(fvhd_handle h, Step* st, const bf16* z, const bf16* w1, 
     if ((rc = make_tmap(h, &td, out, M, c, c, 32, 64)) != FVHD_OK) return rc;
     const dim3 grid((unsigned)(mp.tiles_m < h->num_sms ? mp.tiles_m : h->num_sms));
     const size_t smem = mlp_smem_bytes(c);
+    const bool pdl = h->opt.pdl;
     *st = [=](cudaStream_t s, const RunCtx&) -> cudaError_t {
-        return launch_k(mlp_fused_tcgen05_kernel, grid, dim3(MLP_THREADS), smem, s, tz, tw1, tw2, td, mp);
+        return launch_k(pdl, mlp_fused_tcgen05_kernel, grid, dim3(MLP_THREADS), smem, s, tz, tw1, tw2, td, mp);
     };
-    return FVHD_OK;
-}
-int add_fused_mlp_step(fvhd_handle h, Plan& pl, int unit, const std::string& p, const bf16* z, const bf16* resid, bf16* out, int M, int c) {
-    Step st;
-    int rc = make_fused_mlp_step(h, &st, z, WB(h, p + "fc1.w"), WF(h, p + "fc1.b"), WB(h, p + "fc2.w"), WF(h, p + "fc2.b"), resid, out, M, c);
-    if (rc != FVHD_OK) return rc;
-    pl.add(st, "mlp_fused_tcgen05_kernel", unit, 2.0 * gemm_flops(M, 4 * c, c), 2.0 * (3.0 * M * c + 8.0 * c * c) + 20.0 * c);
     return FVHD_OK;
 }
 
@@ -760,10 +836,29 @@ int make_attention_umma_step(fvhd_handle h, Step* st, const bf16* qkv, bf16* out
     int rc = make_tmap(h, &tm, qkv, (int64_t)batch * N, 3LL * c, 3LL * c, AttU::KT, AttU::HD, CU_TENSOR_MAP_SWIZZLE_64B);
     if (rc != FVHD_OK) return rc;
     const dim3 grid((unsigned)ap.qpairs, (unsigned)(c / AttU::HD), (unsigned)batch);
+    const bool pdl = h->opt.pdl;
     *st = [=](cudaStream_t s, const RunCtx&) -> cudaError_t {
-        return launch_k(attention_umma_kernel, grid, dim3(AttU::THREADS), AttU::SMEM, s, tm, ap);
+        return launch_k(pdl, attention_umma_kernel, grid, dim3(AttU::THREADS), AttU::SMEM, s, tm, ap);
     };
     return FVHD_OK;
+}
+
+// MHSA core on mma.sync (stem_attn_se.cuh): one CTA per (64 queries, head, image).
+int make_attention_mma_step(fvhd_handle h, Step* st, const bf16* qkv, bf16* out, int batch, int N, int c, float scale_log2e) {
+    const dim3 grid((N + 63) / 64, c / 32, batch);
+    const bool pdl = h->opt.pdl;
+    *st = [=](cudaStream_t s, const RunCtx&) -> cudaError_t {
+        return launch_k(pdl, attention_kernel, grid, dim3(128), 0, s, qkv, out, N, c, scale_log2e);
+    };
+    return FVHD_OK;
+}
+
+enum class Attn { Mma, Umma };
+
+// Automatic choice: the tcgen05 / TMEM kernel from 512 tokens (one CTA = 256 queries x 1 head: at N = 256 there are too few
+// CTAs and the mma.sync kernel's finer grid wins -- measured 12.3 vs 10.5 us at batch 1, 86 vs 84 us at batch 32).
+Attn choose_attention(fvhd_handle h, int N) {
+    return (h->opt.attn == 'u' || (h->opt.attn == 'a' && N >= 512)) ? Attn::Umma : Attn::Mma;
 }
 
 // Second-generation fused ConvFFN (convffn.cuh): one CTA per 128-pixel tile, 16 epilogue warps, packed-half GELU, C in {96, 192, 384}.
@@ -780,24 +875,19 @@ int make_convffn2_step_t(fvhd_handle h, Step* st, const bf16* z, const bf16* w1,
     if ((rc = make_tmap(h, &tw1, w1, 4 * C, C, C, MLP_NH)) != FVHD_OK) return rc;
     if ((rc = make_tmap(h, &tw2, w2, C, 4 * C, 4 * C, CfCfg<C>::N2)) != FVHD_OK) return rc;
     const size_t smem = CfCfg<C>::SMEM;
-    // FVHD_CONVFFN_CS=2: 2-CTA clusters sharing the weight stream by TMA multicast (halves each SM's L2 -> smem weight ingest).
-    // Bit-identical and tested, but measured NEUTRAL at batch 32 (C = 384: 303.5 vs 304.0 us, C = 192: 383.7 vs 386.4 us per launch):
-    // the kernel is bound by its MMA1 -> GELU -> MMA2 dependency chain, not by operand ingest.  Default: single CTAs.
-    int cs = 1;
-    { const char* e = getenv("FVHD_CONVFFN_CS"); if (e && (e[0] == '1' || e[0] == '2')) cs = e[0] - '0'; }
+    const bool pdl = h->opt.pdl;
     const int ci = C == 96 ? 0 : C == 192 ? 1 : 2;
-    if (cs == 2 && h->cf_clusters[ci] <= 0) cs = 1;
-    if (cs == 2) {
+    if (h->opt.convffn_cs == 2 && h->cf_clusters[ci] > 0) {     // 2-CTA clusters sharing the weight stream (halves each SM's weight ingest)
         const int want = (mp.tiles_m + 1) / 2;
         const dim3 grid2((unsigned)(2 * (want < h->cf_clusters[ci] ? want : h->cf_clusters[ci])));
         *st = [=](cudaStream_t s, const RunCtx&) -> cudaError_t {
-            return launch_kc(2, convffn_tcgen05_kernel<C, 2>, grid2, dim3(CF_THREADS), smem, s, tz, tw1, tw2, mp);
+            return launch_kc(pdl, 2, convffn_tcgen05_kernel<C, 2>, grid2, dim3(CF_THREADS), smem, s, tz, tw1, tw2, mp);
         };
         return FVHD_OK;
     }
     const dim3 grid((unsigned)(mp.tiles_m < h->num_sms ? mp.tiles_m : h->num_sms));
     *st = [=](cudaStream_t s, const RunCtx&) -> cudaError_t {
-        return launch_k(convffn_tcgen05_kernel<C, 1>, grid, dim3(CF_THREADS), smem, s, tz, tw1, tw2, mp);
+        return launch_k(pdl, convffn_tcgen05_kernel<C, 1>, grid, dim3(CF_THREADS), smem, s, tz, tw1, tw2, mp);
     };
     return FVHD_OK;
 }
@@ -807,13 +897,6 @@ int make_convffn2_step(fvhd_handle h, Step* st, const bf16* z, const bf16* w1, c
     if (c == 192) return make_convffn2_step_t<192>(h, st, z, w1, b1, w2, w2_f16, b2, resid, out, M);
     if (c == 384) return make_convffn2_step_t<384>(h, st, z, w1, b1, w2, w2_f16, b2, resid, out, M);
     return fail(h, FVHD_ERR_INVALID, "convffn_tcgen05_kernel exists for C in {96, 192, 384}, got %d", c);
-}
-int add_convffn2_step(fvhd_handle h, Plan& pl, int unit, const std::string& p, const bf16* z, const bf16* resid, bf16* out, int M, int c) {
-    Step st;
-    int rc = make_convffn2_step(h, &st, z, WB(h, p + "fc1.w"), WF(h, p + "fc1.b"), h->wptr.at(p + "fc2.wh"), 1, WF(h, p + "fc2.b"), resid, out, M, c);
-    if (rc != FVHD_OK) return rc;
-    pl.add(st, "convffn_tcgen05_kernel", unit, 2.0 * gemm_flops(M, 4 * c, c), 2.0 * (3.0 * M * c + 8.0 * c * c) + 20.0 * c);
-    return FVHD_OK;
 }
 
 // Stage-2 ConvFFN (C = 384): one 4-CTA cluster per 128-pixel tile, hidden split across the cluster, DSMEM reduction.
@@ -831,19 +914,31 @@ int make_cluster_mlp_step(fvhd_handle h, Step* st, const bf16* z, const bf16* w1
     if ((rc = make_tmap(h, &tw2, w2, c, 4 * c, 4 * c, MLPC_NHALF)) != FVHD_OK) return rc;
     const int clusters = mp.tiles_m < h->mlpc_clusters ? mp.tiles_m : h->mlpc_clusters;
     const dim3 grid((unsigned)(clusters * MLPC_CS));
+    const bool pdl = h->opt.pdl;
     *st = [=](cudaStream_t s, const RunCtx&) -> cudaError_t {
-        return launch_kc(MLPC_CS, mlp_cluster_tcgen05_kernel, grid, dim3(MLPC_THREADS), MLPC_SMEM, s, tz, tw1, tw2, mp);
+        return launch_kc(pdl, MLPC_CS, mlp_cluster_tcgen05_kernel, grid, dim3(MLPC_THREADS), MLPC_SMEM, s, tz, tw1, tw2, mp);
     };
     return FVHD_OK;
 }
-int add_cluster_mlp_step(fvhd_handle h, Plan& pl, int unit, const std::string& p, const bf16* z, const bf16* resid, bf16* out, int M) {
-    const int c = MLPC_C;
-    Step st;
-    int rc = make_cluster_mlp_step(h, &st, z, WB(h, p + "fc1.w"), WF(h, p + "fc1.b"), WB(h, p + "fc2.w"), WF(h, p + "fc2.b"), resid, out, M, nullptr);
-    if (rc != FVHD_OK) return rc;
-    pl.add(st, "mlp_cluster_tcgen05_kernel", unit, 2.0 * gemm_flops(M, 4 * c, c), 2.0 * (3.0 * M * c + 8.0 * c * c) + 20.0 * c);
-    return FVHD_OK;
+
+// The ConvFFN of a RepMixer block over M pixels of C channels.
+enum class ConvFfn { Gen2, Fused, Cluster, TwoGemms };
+
+ConvFfn choose_convffn(fvhd_handle h, int M, int c) {
+    const Options& o = h->opt;
+    // the 4-CTA cluster kernel at small batches only: beyond two tiles per resident cluster the two plain GEMMs fill the machine better
+    // (measured: batch 1 0.71 vs 0.91 ms for the 24 blocks, batch 4 2.23 vs 2.15 ms, batch 8 4.28 vs 3.67 ms)
+    const bool few_tiles = c == MLPC_C && o.cluster_mlp && h->mlpc_clusters > 0 && (M + GEMM_BM - 1) / GEMM_BM <= 2 * h->mlpc_clusters;
+    // second-generation single-CTA kernel: every C, any batch (stage 2 at batch <= 2 keeps the 4-CTA cluster kernel: 32 tiles per
+    // image cannot fill 148 SMs one tile per CTA)
+    if (o.fused_mlp && o.convffn_gen == 2 && !few_tiles) return ConvFfn::Gen2;
+    if (o.fused_mlp && c <= 192) return ConvFfn::Fused;
+    return few_tiles ? ConvFfn::Cluster : ConvFfn::TwoGemms;
 }
+
+enum class Stem { Gen1, Gen2 };
+
+Stem choose_stem(fvhd_handle h) { return h->opt.stem_gen == 1 ? Stem::Gen1 : Stem::Gen2; }
 
 int build_plan(fvhd_handle h, int batch, Plan& pl) {
     pl = Plan();
@@ -854,6 +949,7 @@ int build_plan(fvhd_handle h, int batch, Plan& pl) {
     bf16* cur = bf.X0;
     bf16* nxt = bf.X1;
     int rc;
+    const bool pdl = h->opt.pdl;
     const size_t nunits = h->units.size();
     for (size_t ui = 0; ui < nunits; ++ui) {
         const UnitDesc& u = h->units[ui];
@@ -874,19 +970,19 @@ int build_plan(fvhd_handle h, int batch, Plan& pl) {
             bf16* t0 = bf.T1;
             const double stem_flops = 2.0 * batch * ((double)(R / 2) * (R / 2) * 96 * 27 + (double)(R / 4) * (R / 4) * 96 * 9);
             const double stem_bytes = (double)batch * (3.0 * R * R * 2 + (double)(R / 4) * (R / 4) * 96 * 2);
-            if (g_stem_gen == 2) {
+            if (choose_stem(h) == Stem::Gen2) {
                 const int n_tiles = tiles * tiles * batch;
                 const dim3 grid2((unsigned)std::min(n_tiles, 3 * h->num_sms));
                 pl.add([=](cudaStream_t s, const RunCtx& ctx) -> cudaError_t {
-                    if (ctx.img_dtype == FVHD_F32) return launch_k(stem2_kernel<float>, grid2, dim3(Stem2::THREADS), Stem2::SMEM, s, io, t0, w0, b0, w1, b1, R, tiles, n_tiles);
-                    if (ctx.img_dtype == FVHD_F16) return launch_k(stem2_kernel<__half>, grid2, dim3(Stem2::THREADS), Stem2::SMEM, s, io, t0, w0, b0, w1, b1, R, tiles, n_tiles);
-                    return launch_k(stem2_kernel<bf16>, grid2, dim3(Stem2::THREADS), Stem2::SMEM, s, io, t0, w0, b0, w1, b1, R, tiles, n_tiles);
+                    if (ctx.img_dtype == FVHD_F32) return launch_k(pdl, stem2_kernel<float>, grid2, dim3(Stem2::THREADS), Stem2::SMEM, s, io, t0, w0, b0, w1, b1, R, tiles, n_tiles);
+                    if (ctx.img_dtype == FVHD_F16) return launch_k(pdl, stem2_kernel<__half>, grid2, dim3(Stem2::THREADS), Stem2::SMEM, s, io, t0, w0, b0, w1, b1, R, tiles, n_tiles);
+                    return launch_k(pdl, stem2_kernel<bf16>, grid2, dim3(Stem2::THREADS), Stem2::SMEM, s, io, t0, w0, b0, w1, b1, R, tiles, n_tiles);
                 }, "stem2_kernel", U, stem_flops, stem_bytes);
             } else {
             pl.add([=](cudaStream_t s, const RunCtx& ctx) -> cudaError_t {
-                if (ctx.img_dtype == FVHD_F32) return launch_k(stem_kernel<float>, grid, dim3(STEM_THREADS), STEM_SMEM, s, io, t0, w0, b0, w1, b1, R, tiles);
-                if (ctx.img_dtype == FVHD_F16) return launch_k(stem_kernel<__half>, grid, dim3(STEM_THREADS), STEM_SMEM, s, io, t0, w0, b0, w1, b1, R, tiles);
-                return launch_k(stem_kernel<bf16>, grid, dim3(STEM_THREADS), STEM_SMEM, s, io, t0, w0, b0, w1, b1, R, tiles);
+                if (ctx.img_dtype == FVHD_F32) return launch_k(pdl, stem_kernel<float>, grid, dim3(STEM_THREADS), STEM_SMEM, s, io, t0, w0, b0, w1, b1, R, tiles);
+                if (ctx.img_dtype == FVHD_F16) return launch_k(pdl, stem_kernel<__half>, grid, dim3(STEM_THREADS), STEM_SMEM, s, io, t0, w0, b0, w1, b1, R, tiles);
+                return launch_k(pdl, stem_kernel<bf16>, grid, dim3(STEM_THREADS), STEM_SMEM, s, io, t0, w0, b0, w1, b1, R, tiles);
             }, "stem_kernel", U, stem_flops, stem_bytes);
             }
             if ((rc = add_gemm(h, pl, U, t0, 96, WB(h, "stem.w2"), WF(h, "stem.b2"), nullptr, 0, out, 96, M, 96, 96, 1)) != FVHD_OK) return rc;
@@ -895,74 +991,23 @@ int build_plan(fvhd_handle h, int batch, Plan& pl) {
         }
         case 1: {   // RepMixerBlock: fused dw3x3 -> y, dw7x7(+BN) -> z ; fc1+GELU ; fc2 (+layer scale folded) + y
             const float *w3 = WF(h, p + "mix.w"), *b3 = WF(h, p + "mix.b"), *w7 = WF(h, p + "dw.w"), *b7 = WF(h, p + "dw.b");
-            // default: 16x16 tiles with the 7x7 on the tensor cores (mixer_tc.cuh).  FVHD_MIX_TILE selects the FMA-pipe variants
-            // of dwconv.cuh instead: 'a' = their old automatic choice, '1' = 16x16/256 thr, '8' = 8x16/128 thr, '5' = 16x16/512 thr.
-            const long ctas16 = (long)((W + 15) / 16) * ((H + 15) / 16) * (c / DW_CG) * batch;
-            if (g_mixer_mode == '2' && !getenv("FVHD_MIX_TILE") && c % MixT2::CG == 0) {
-                // both convs on mma.sync, 16 channels per CTA (mixer_tc2.cuh)
-                const int tx2 = (W + MixT2::TOW - 1) / MixT2::TOW, ty2 = (H + MixT2::TOH - 1) / MixT2::TOH;
-                const dim3 grid2(tx2 * ty2, c / MixT2::CG, batch);
-                CUtensorMap tm2;
-                if ((rc = make_tmap_nhwc(h, &tm2, in, batch, H, W, c, MixT2::XP, MixT2::XH, MixT2::CG)) != FVHD_OK) return rc;
-                bf16 *y2 = bf.Y, *z2 = bf.Z;
-                pl.add([=](cudaStream_t s, const RunCtx&) -> cudaError_t {
-                    return launch_k(repmixer_tc2_kernel, grid2, dim3(MixT2::NT), MixT2::SMEM, s, tm2, y2, z2, w3, b3, w7, b7, H, W, c, tx2);
-                }, "repmixer_tc2_kernel", U, 2.0 * Md * c * 58, 3.0 * Md * c * 2);
-            } else if (g_mixer_mode == 'u' && !getenv("FVHD_MIX_TILE")) {
-                Step ms;
-                if ((rc = make_mixer_umma_step(h, &ms, in, bf.Y, bf.Z, w3, b3, w7, b7, batch, H, W, c)) != FVHD_OK) return rc;
-                pl.add(ms, "repmixer_umma_kernel", U, 2.0 * Md * c * 58, 3.0 * Md * c * 2);
-            } else if (g_mixer_mode == 'z' && !getenv("FVHD_MIX_TILE") &&
-                       ((long)batch * ((W + MixZ::ZC - 1) / MixZ::ZC) * ((H + MixZ::ZR - 1) / MixZ::ZR) * (c / MixZ::CG) >= h->num_sms || c % DW_CG != 0 ||
-                        getenv("FVHD_MIXER") != nullptr)) {
-                // Toeplitz tcgen05 mixer whenever there is at least one 64 x 32 x 8 item per SM; below that (stage 2 of a single
-                // 1024-px image: 96 items) the finer-grained mma.sync kernel of mixer_tc.cuh has the shorter critical path
-                // (16 vs 20 us per launch at batch 1).  An explicit FVHD_MIXER=z forces it everywhere.
-                Step ms;
-                if ((rc = make_mixer_tz_step(h, &ms, in, bf.Y, bf.Z, w3, b3, w7, b7, batch, H, W, c)) != FVHD_OK) return rc;
-                pl.add(ms, "repmixer_tz_kernel", U, 2.0 * Md * c * 58, 3.0 * Md * c * 2);
-            } else {
-            bool small = false, wide = false, tc = g_mixer_mode != 'f';
-            { const char* e = getenv("FVHD_MIX_TILE");
-              if (e && e[0] == 'a') { tc = false; small = ctas16 < 2L * h->num_sms; }
-              else if (e && e[0] == '8') { tc = false; small = true; }
-              else if (e && e[0] == '1') { tc = false; }
-              else if (e && e[0] == '5') { tc = false; wide = true; } }
-            const int TH = small ? 8 : 16;
-            const int tx = (W + 15) / 16, ty = (H + TH - 1) / TH;
-            const dim3 grid(tx * ty, c / DW_CG, batch);
-            // mixer_tc: persistent CTAs, ~two per SM in total, each bound to one 32-channel group and walking that group's (image, tile) items
-            int per_group = (2 * h->num_sms) / (c / DW_CG);       // floor: a CTA beyond the resident slots would run its whole item loop as a second wave
-            if (per_group < 1) per_group = 1;
-            if (per_group > tx * ty * batch) per_group = tx * ty * batch;
-            const dim3 grid_tc(per_group, c / DW_CG, 1);
             bf16 *y = bf.Y, *z = bf.Z;
-            CUtensorMap tmx;
-            if ((rc = make_tmap_nhwc(h, &tmx, in, batch, H, W, c, small ? MixCfgT<8, 16>::XP : MixCfgT<16, 16>::XP,
-                                     small ? MixCfgT<8, 16>::XH : MixCfgT<16, 16>::XH)) != FVHD_OK) return rc;
-            static_assert(MixTc::XP == MixCfgT<16, 16>::XP && MixTc::XH == MixCfgT<16, 16>::XH, "same TMA box for both 16x16 kernels");
-            pl.add([=](cudaStream_t s, const RunCtx&) -> cudaError_t {
-                if (tc) return launch_k(repmixer_tc_kernel, grid_tc, dim3(MixTc::NT), MixTc::SMEM, s, tmx, y, z, w3, b3, w7, b7, H, W, c, tx, batch);
-                if (wide) return launch_k(repmixer_dw_kernel<16, 16, 512, 6, 4, 2>, grid, dim3(512), MixCfgT<16, 16>::SMEM, s, tmx, y, z, w3, b3, w7, b7, H, W, c, tx);
-                if (small) return launch_k(repmixer_dw_kernel<8, 16, 128>, grid, dim3(128), MixCfgT<8, 16>::SMEM, s, tmx, y, z, w3, b3, w7, b7, H, W, c, tx);
-                return launch_k(repmixer_dw_kernel<16, 16, 256>, grid, dim3(256), MixCfgT<16, 16>::SMEM, s, tmx, y, z, w3, b3, w7, b7, H, W, c, tx);
-            }, tc ? "repmixer_tc_kernel" : "repmixer_dw_kernel", U, 2.0 * Md * c * 58, 3.0 * Md * c * 2);
+            const auto& mk = kMixers[(int)choose_mixer(h, batch, H, W, c)];
+            Step ms;
+            if ((rc = mk.make(h, &ms, in, y, z, w3, b3, w7, b7, batch, H, W, c)) != FVHD_OK) return rc;
+            pl.add(ms, mk.kernel, U, 2.0 * Md * c * 58, 3.0 * Md * c * 2);
+            const bf16 *w1 = WB(h, p + "fc1.w"), *w2 = WB(h, p + "fc2.w");
+            const float *b1 = WF(h, p + "fc1.b"), *b2 = WF(h, p + "fc2.b");
+            Step fs;
+            const char* fk = nullptr;       // the fused kernels' name; two GEMMs add their own steps
+            switch (choose_convffn(h, M, c)) {
+            case ConvFfn::Gen2: rc = make_convffn2_step(h, &fs, z, w1, b1, h->wptr.at(p + "fc2.wh"), 1, b2, y, out, M, c); fk = "convffn_tcgen05_kernel"; break;
+            case ConvFfn::Fused: rc = make_fused_mlp_step(h, &fs, z, w1, b1, w2, b2, y, out, M, c); fk = "mlp_fused_tcgen05_kernel"; break;
+            case ConvFfn::Cluster: rc = make_cluster_mlp_step(h, &fs, z, w1, b1, w2, b2, y, out, M, nullptr); fk = "mlp_cluster_tcgen05_kernel"; break;
+            case ConvFfn::TwoGemms: rc = add_convffn_steps(h, pl, U, p, bf, z, y, out, M, c); break;
             }
-            bf16 *y = bf.Y, *z = bf.Z;
-            const bool few_tiles = c == MLPC_C && g_use_cluster_mlp && h->mlpc_clusters > 0 && (M + GEMM_BM - 1) / GEMM_BM <= 2 * h->mlpc_clusters;
-            if (g_use_fused_mlp && g_convffn_gen == 2 && !few_tiles) {
-                // second-generation single-CTA kernel: every C, any batch (stage 2 at batch <= 2 keeps the 4-CTA cluster kernel:
-                // 32 tiles per image cannot fill 148 SMs one tile per CTA)
-                if ((rc = add_convffn2_step(h, pl, U, p, z, y, out, M, c)) != FVHD_OK) return rc;
-            } else if (g_use_fused_mlp && c <= 192) {
-                if ((rc = add_fused_mlp_step(h, pl, U, p, z, y, out, M, c)) != FVHD_OK) return rc;
-            } else if (g_use_cluster_mlp && c == MLPC_C && h->mlpc_clusters > 0 && (M + GEMM_BM - 1) / GEMM_BM <= 2 * h->mlpc_clusters) {
-                // small batches only: beyond two tiles per resident cluster the two plain GEMMs fill the machine better
-                // (measured: batch 1 0.71 vs 0.91 ms for the 24 blocks, batch 4 2.23 vs 2.15 ms, batch 8 4.28 vs 3.67 ms)
-                if ((rc = add_cluster_mlp_step(h, pl, U, p, z, y, out, M)) != FVHD_OK) return rc;
-            } else {
-                if ((rc = add_convffn_steps(h, pl, U, p, bf, z, y, out, M, c)) != FVHD_OK) return rc;
-            }
+            if (rc != FVHD_OK) return rc;
+            if (fk) pl.add(fs, fk, U, 2.0 * gemm_flops(M, 4 * c, c), 2.0 * (3.0 * M * c + 8.0 * c * c) + 20.0 * c);
             break;
         }
         case 2: {   // PatchEmbed: dw7x7 s2 (x2 channels) + GELU ; 1x1 + GELU
@@ -980,23 +1025,15 @@ int build_plan(fvhd_handle h, int batch, Plan& pl) {
             const int lngrid = (M + 7) / 8;
             if (c != 768 && c != 1536) return fail(h, FVHD_ERR_INVALID, "LayerNorm kernel expects C in {768,1536}, got %d", c);
             pl.add([=](cudaStream_t s, const RunCtx&) -> cudaError_t {
-                if (c == 768) return launch_k(layernorm_channel_kernel<3>, dim3(lngrid), dim3(256), 0, s, in, t1, lw, lb, M, 1e-5f);
-                return launch_k(layernorm_channel_kernel<6>, dim3(lngrid), dim3(256), 0, s, in, t1, lw, lb, M, 1e-5f);
+                if (c == 768) return launch_k(pdl, layernorm_channel_kernel<3>, dim3(lngrid), dim3(256), 0, s, in, t1, lw, lb, M, 1e-5f);
+                return launch_k(pdl, layernorm_channel_kernel<6>, dim3(lngrid), dim3(256), 0, s, in, t1, lw, lb, M, 1e-5f);
             }, "layernorm_channel_kernel", U, 0.0, 4.0 * Md * c);
             if ((rc = add_gemm(h, pl, U, t1, c, WB(h, p + "qkv.w"), nullptr, nullptr, 0, qkv, 3 * c, M, 3 * c, c, 0)) != FVHD_OK) return rc;
             const float sl2 = 0.17677669529663687f * 1.4426950408889634f;   // 32^-0.5 * log2(e)
-            // auto: tcgen05 / TMEM kernel from 512 tokens (one CTA = 256 queries x 1 head: at N = 256 there are too few CTAs and the
-            // mma.sync kernel's finer grid wins -- measured 12.3 vs 10.5 us at batch 1, 86 vs 84 us at batch 32)
-            if (g_attn_mode == 'u' || (g_attn_mode == 'a' && N >= 512)) {       // tcgen05 / TMEM flash attention (attention_umma.cuh)
-                Step as;
-                if ((rc = make_attention_umma_step(h, &as, qkv, t1, batch, N, c, sl2)) != FVHD_OK) return rc;
-                pl.add(as, "attention_umma_kernel", U, 4.0 * batch * (double)N * N * c, 8.0 * Md * c);
-            } else {
-                const dim3 agrid((N + 63) / 64, c / 32, batch);
-                pl.add([=](cudaStream_t s, const RunCtx&) -> cudaError_t {
-                    return launch_k(attention_kernel, agrid, dim3(128), 0, s, qkv, t1, N, c, sl2);
-                }, "attention_kernel", U, 4.0 * batch * (double)N * N * c, 8.0 * Md * c);
-            }
+            const bool umma = choose_attention(h, N) == Attn::Umma;
+            Step as;
+            if ((rc = (umma ? make_attention_umma_step : make_attention_mma_step)(h, &as, qkv, t1, batch, N, c, sl2)) != FVHD_OK) return rc;
+            pl.add(as, umma ? "attention_umma_kernel" : "attention_kernel", U, 4.0 * batch * (double)N * N * c, 8.0 * Md * c);
             if ((rc = add_gemm(h, pl, U, t1, c, WB(h, p + "proj.w"), WF(h, p + "proj.b"), in, c, x1, c, M, c, c, 0)) != FVHD_OK) return rc;
             { Step ds; if ((rc = make_dw7_step(h, &ds, x1, bf.Z, WF(h, p + "dw.w"), WF(h, p + "dw.b"), batch, H, W, c)) != FVHD_OK) return rc; pl.add(ds, "dwconv_kernel<7,1,1>", U, 2.0 * Md * c * 49, 4.0 * Md * c); }
             if ((rc = add_convffn_steps(h, pl, U, p, bf, bf.Z, x1, out, M, c)) != FVHD_OK) return rc;
@@ -1011,13 +1048,13 @@ int build_plan(fvhd_handle h, int batch, Plan& pl) {
             const float *br = WF(h, p + "se.r.b"), *be = WF(h, p + "se.e.b");
             bf16* dst = last ? nullptr : out;
             pl.add([=](cudaStream_t s, const RunCtx&) -> cudaError_t {
-                return launch_k(se_pool_kernel, dim3(3072 / 64, batch), dim3(256), 0, s, cexp, pooled, HW, 3072);
+                return launch_k(pdl, se_pool_kernel, dim3(3072 / 64, batch), dim3(256), 0, s, cexp, pooled, HW, 3072);
             }, "se_pool_kernel", U, 0.0, 2.0 * Md * 3072);
             pl.add([=](cudaStream_t s, const RunCtx&) -> cudaError_t {
-                return launch_k(se_reduce_kernel, dim3(kSeRd / 8, batch), dim3(256), 0, s, pooled, wr, br, sr, 3072, kSeRd);
+                return launch_k(pdl, se_reduce_kernel, dim3(kSeRd / 8, batch), dim3(256), 0, s, pooled, wr, br, sr, 3072, kSeRd);
             }, "se_reduce_kernel", U, 2.0 * batch * 3072 * kSeRd, 2.0 * 3072 * kSeRd);
             pl.add([=](cudaStream_t s, const RunCtx&) -> cudaError_t {
-                return launch_k(se_expand_scale_gelu_kernel, dim3(3072 / 64, batch), dim3(256), 0, s, cexp, sr, we, be, dst, io, HW, 3072, kSeRd);
+                return launch_k(pdl, se_expand_scale_gelu_kernel, dim3(3072 / 64, batch), dim3(256), 0, s, cexp, sr, we, be, dst, io, HW, 3072, kSeRd);
             }, "se_expand_scale_gelu_kernel", U, 2.0 * batch * 3072 * kSeRd, 4.0 * Md * 3072 + 2.0 * 3072 * kSeRd);
             break;
         }
@@ -1067,6 +1104,13 @@ int check_ready(fvhd_handle h, int batch) {
 
 size_t dtype_size(int dt) { return dt == FVHD_F32 ? 4 : 2; }
 
+// One stand-alone step on `stream` (the single-kernel entries).
+int launch_step(fvhd_handle h, const Step& s, void* stream, const char* what) {
+    cudaError_t e = s(reinterpret_cast<cudaStream_t>(stream), RunCtx{});
+    if (e != cudaSuccess) return fail(h, FVHD_ERR_CUDA, "%s launch failed: %s", what, cudaGetErrorString(e));
+    return FVHD_OK;
+}
+
 // Run steps [s0, s1) of a plan (direct launches).
 int run_steps(fvhd_handle h, Plan& pl, int s0, int s1, cudaStream_t st, const RunCtx& ctx) {
     for (int i = s0; i < s1; ++i) {
@@ -1082,7 +1126,7 @@ int set_io(fvhd_handle h, Plan& pl, cudaStream_t st, const void* images, void* f
     if (peers) pl_peers = *peers;
     ScatterList sc{};
     if (scatter) sc = *scatter;
-    cudaError_t e = launch_k(set_io_kernel, dim3(1), dim3(FVHD_MAX_SCATTER), 0, st, pl.io, images, final_out, tokens_out, final_image_stride, pl_peers, sc);
+    cudaError_t e = launch_k(h->opt.pdl, set_io_kernel, dim3(1), dim3(FVHD_MAX_SCATTER), 0, st, pl.io, images, final_out, tokens_out, final_image_stride, pl_peers, sc);
     if (e != cudaSuccess) return fail(h, FVHD_ERR_CUDA, "set_io_kernel launch failed: %s", cudaGetErrorString(e));
     return FVHD_OK;
 }
@@ -1091,7 +1135,7 @@ int launch_copy_tokens(fvhd_handle h, Plan& pl, cudaStream_t st, const bf16* src
     const size_t n16 = bytes / 16;
     int blocks = (int)((n16 + 255) / 256);
     if (blocks > 1184) blocks = 1184;
-    cudaError_t e = launch_k(copy_tokens_kernel, dim3(blocks), dim3(256), 0, st, reinterpret_cast<const uint4*>(src), pl.io, n16);
+    cudaError_t e = launch_k(h->opt.pdl, copy_tokens_kernel, dim3(blocks), dim3(256), 0, st, reinterpret_cast<const uint4*>(src), pl.io, n16);
     if (e != cudaSuccess) return fail(h, FVHD_ERR_CUDA, "copy_tokens_kernel launch failed: %s", cudaGetErrorString(e));
     return FVHD_OK;
 }
@@ -1102,7 +1146,7 @@ int run_forward(fvhd_handle h, Plan& pl, cudaStream_t st, const RunCtx& ctx, int
     int rc;
     cudaStreamCaptureStatus cs = cudaStreamCaptureStatusNone;
     cudaStreamIsCapturing(st, &cs);
-    if (!h->use_graph || cs != cudaStreamCaptureStatusNone) {
+    if (!h->opt.graph || cs != cudaStreamCaptureStatusNone) {
         if ((rc = run_steps(h, pl, 0, last_step, st, ctx)) != FVHD_OK) return rc;
         if (tok_src) return launch_copy_tokens(h, pl, st, tok_src, tok_bytes);
         return FVHD_OK;
@@ -1149,6 +1193,7 @@ int build_llm_plan(fvhd_handle h, LlmState* S, int L, Plan& pl) {
     const int ln_grid = (L + 7) / 8;
     const float sl2 = 1.4426950408889634f / sqrtf((float)D);
     const float2* rope = S->rope;
+    const bool pdl = h->opt.pdl;
     auto add_gemm_l = [&](const bf16* A, int lda, const void* W, const void* bias, const bf16* resid, bf16* Dp, int M, int N, int K) -> int {
         Step g;
         int r = make_gemm_step(h, &g, nullptr, 1, A, lda, (const bf16*)W, (const float*)bias, resid, N, Dp, N, M, N, K, 0);
@@ -1164,32 +1209,30 @@ int build_llm_plan(fvhd_handle h, LlmState* S, int L, Plan& pl) {
         bf16* vc = S->vc + (size_t)l * c.max_seq * c.kv_heads * D;
         const bf16* xin = xc;
         const float eps = c.rms_eps;
-        pl.add([=](cudaStream_t s, const RunCtx&) -> cudaError_t { return launch_k(rmsnorm_kernel, dim3(ln_grid), dim3(256), 0, s, xin, xn, ln1, L, H, eps); },
+        pl.add([=](cudaStream_t s, const RunCtx&) -> cudaError_t { return launch_k(pdl, rmsnorm_kernel, dim3(ln_grid), dim3(256), 0, s, xin, xn, ln1, L, H, eps); },
                "rmsnorm_kernel", 0, 0.0, 4.0 * L * H);
         if ((rc = add_gemm_l(xn, H, w[1], w[2], nullptr, qkv, L, NQ, H)) != FVHD_OK) return rc;
         const int heads = c.heads, kvh = c.kv_heads;
-        const char* attn_env = getenv("FVHD_LLM_ATTN");      // read when a plan (one per sequence length) is built
-        const bool attn_fma = attn_env && attn_env[0] == 'f';
-        if (attn_fma) {      // FVHD_LLM_ATTN=f: the FMA-pipe kernel (first version; kept for A/B)
+        if (h->opt.llm_attn_fma) {      // FVHD_LLM_ATTN=f: the FMA-pipe kernel (first version; kept for A/B)
             const dim3 agrid((L + LLM_ATTN_QB - 1) / LLM_ATTN_QB, heads);
             pl.add([=](cudaStream_t s, const RunCtx&) -> cudaError_t {
-                       if (D == 64) return launch_k(causal_attn_kernel<64>, agrid, dim3(LLM_ATTN_THREADS), LlmAttnSmem<64>::BYTES, s, (const bf16*)qkv, att, rope, kc, vc, L, heads, kvh, sl2);
-                       return launch_k(causal_attn_kernel<128>, agrid, dim3(LLM_ATTN_THREADS), LlmAttnSmem<128>::BYTES, s, (const bf16*)qkv, att, rope, kc, vc, L, heads, kvh, sl2);
+                       if (D == 64) return launch_k(pdl, causal_attn_kernel<64>, agrid, dim3(LLM_ATTN_THREADS), LlmAttnSmem<64>::BYTES, s, (const bf16*)qkv, att, rope, kc, vc, L, heads, kvh, sl2);
+                       return launch_k(pdl, causal_attn_kernel<128>, agrid, dim3(LLM_ATTN_THREADS), LlmAttnSmem<128>::BYTES, s, (const bf16*)qkv, att, rope, kc, vc, L, heads, kvh, sl2);
                    }, "causal_attn_kernel", 0, 2.0 * (double)L * L * HD, 2.0 * L * (NQ + HD));
         } else {
             const dim3 agrid((L + LLM_MMA_QB - 1) / LLM_MMA_QB, heads);
             pl.add([=](cudaStream_t s, const RunCtx&) -> cudaError_t {
-                       if (D == 64) return launch_k(causal_attn_mma_kernel<64>, agrid, dim3(LLM_MMA_THREADS), LlmAttnMmaSmem<64>::BYTES, s, (const bf16*)qkv, att, rope, kc, vc, L, heads, kvh, sl2);
-                       return launch_k(causal_attn_mma_kernel<128>, agrid, dim3(LLM_MMA_THREADS), LlmAttnMmaSmem<128>::BYTES, s, (const bf16*)qkv, att, rope, kc, vc, L, heads, kvh, sl2);
+                       if (D == 64) return launch_k(pdl, causal_attn_mma_kernel<64>, agrid, dim3(LLM_MMA_THREADS), LlmAttnMmaSmem<64>::BYTES, s, (const bf16*)qkv, att, rope, kc, vc, L, heads, kvh, sl2);
+                       return launch_k(pdl, causal_attn_mma_kernel<128>, agrid, dim3(LLM_MMA_THREADS), LlmAttnMmaSmem<128>::BYTES, s, (const bf16*)qkv, att, rope, kc, vc, L, heads, kvh, sl2);
                    }, "causal_attn_mma_kernel", 0, 2.0 * (double)L * L * HD, 2.0 * L * (NQ + HD));
         }
         if ((rc = add_gemm_l(att, HD, w[3], nullptr, xc, xx, L, H, HD)) != FVHD_OK) return rc;
         const bf16* x2 = xx;
-        pl.add([=](cudaStream_t s, const RunCtx&) -> cudaError_t { return launch_k(rmsnorm_kernel, dim3(ln_grid), dim3(256), 0, s, x2, xn, ln2, L, H, eps); },
+        pl.add([=](cudaStream_t s, const RunCtx&) -> cudaError_t { return launch_k(pdl, rmsnorm_kernel, dim3(ln_grid), dim3(256), 0, s, x2, xn, ln2, L, H, eps); },
                "rmsnorm_kernel", 0, 0.0, 4.0 * L * H);
         if ((rc = add_gemm_l(xn, H, w[5], nullptr, nullptr, gu, L, 2 * I, H)) != FVHD_OK) return rc;
         const int sgrid = (int)std::min<long>(((long)L * (I / 8) + 255) / 256, 1184);
-        pl.add([=](cudaStream_t s, const RunCtx&) -> cudaError_t { return launch_k(silu_mul_kernel, dim3(sgrid), dim3(256), 0, s, (const bf16*)gu, hm, L, I); },
+        pl.add([=](cudaStream_t s, const RunCtx&) -> cudaError_t { return launch_k(pdl, silu_mul_kernel, dim3(sgrid), dim3(256), 0, s, (const bf16*)gu, hm, L, I); },
                "silu_mul_kernel", 0, 0.0, 6.0 * L * I);
         if ((rc = add_gemm_l(hm, I, w[6], nullptr, xx, S->x2, L, H, I)) != FVHD_OK) return rc;
         xc = S->x2;                              // the input buffer x0 is only ever read: a prefill can be replayed
@@ -1201,10 +1244,10 @@ int build_llm_plan(fvhd_handle h, LlmState* S, int L, Plan& pl) {
     int* tok = S->token;
     const float eps = c.rms_eps;
     const int V = c.vocab;
-    pl.add([=](cudaStream_t s, const RunCtx&) -> cudaError_t { return launch_k(rmsnorm_kernel, dim3(1), dim3(256), 0, s, last, xn, fn, 1, H, eps); },
+    pl.add([=](cudaStream_t s, const RunCtx&) -> cudaError_t { return launch_k(pdl, rmsnorm_kernel, dim3(1), dim3(256), 0, s, last, xn, fn, 1, H, eps); },
            "rmsnorm_kernel", 0, 0.0, 4.0 * H);
     if ((rc = add_gemm_l(xn, H, lm, nullptr, nullptr, logits, 1, V, H)) != FVHD_OK) return rc;
-    pl.add([=](cudaStream_t s, const RunCtx&) -> cudaError_t { return launch_k(argmax_kernel, dim3(1), dim3(1024), 0, s, (const bf16*)logits, V, tok); },
+    pl.add([=](cudaStream_t s, const RunCtx&) -> cudaError_t { return launch_k(pdl, argmax_kernel, dim3(1), dim3(1024), 0, s, (const bf16*)logits, V, tok); },
            "argmax_kernel", 0, 0.0, 2.0 * V);
     return FVHD_OK;
 }
@@ -1232,6 +1275,7 @@ int fvhd_create(const fvhd_config* cfg, fvhd_handle* out) {
     if (cfg->max_batch < 1) return fail(nullptr, FVHD_ERR_INVALID, "max_batch must be >= 1");
     fvhd_handle h = new fvhd_handle_s();
     h->cfg = *cfg;
+    h->opt = read_options();
     h->R = cfg->image_size;
     h->ntok = (cfg->image_size / FVHD_PATCH) * (cfg->image_size / FVHD_PATCH);
     build_arch(h);
@@ -1332,12 +1376,7 @@ int fvhd_launches_per_forward(fvhd_handle h, int batch) {
         for (const UnitDesc& u : h->units) {
             switch (u.kind) {
             case 0: steps += 2; break;
-            case 1: {
-                const int tiles_m = (bc * u.hout * u.wout + GEMM_BM - 1) / GEMM_BM;
-                steps += ((g_use_fused_mlp && (u.cin <= 192 || g_convffn_gen == 2)) ||
-                          (g_use_cluster_mlp && u.cin == MLPC_C && h->mlpc_clusters > 0 && tiles_m <= 2 * h->mlpc_clusters)) ? 2 : 3;
-                break;
-            }
+            case 1: steps += choose_convffn(h, bc * u.hout * u.wout, u.cin) == ConvFfn::TwoGemms ? 3 : 2; break;   // mixer + ConvFFN
             case 2: steps += 2; break;
             case 3: steps += 1; break;
             case 4: steps += 7; break;
@@ -1634,13 +1673,14 @@ static int preprocess_impl(fvhd_handle h, cudaStream_t st, const void* rgb, int 
         h->rs_tmp_bytes = tmp_bytes;
     }
     fvhd_handle_s::RsTable tx{}, ty{};
+    const bool pdl = h->opt.pdl;
     const dim3 g1((ow + 127) / 128, Hs);
     cudaError_t e;
     if (ow != Ws) {
         if ((rc = rs_get_table(h, Ws, ow, &tx)) != FVHD_OK) return rc;
-        e = launch_k(resample_h_kernel, g1, dim3(128), 0, st, src, H, W, offy, offx, Ws, h->rs_tmp, ow, (const int*)tx.bounds, (const int*)tx.kk, tx.ksize);
+        e = launch_k(pdl, resample_h_kernel, g1, dim3(128), 0, st, src, H, W, offy, offx, Ws, h->rs_tmp, ow, (const int*)tx.bounds, (const int*)tx.kk, tx.ksize);
     } else {
-        e = launch_k(pad_copy_kernel, g1, dim3(128), 0, st, src, H, W, offy, offx, h->rs_tmp, ow);
+        e = launch_k(pdl, pad_copy_kernel, g1, dim3(128), 0, st, src, H, W, offy, offx, h->rs_tmp, ow);
     }
     if (e != cudaSuccess) return fail(h, FVHD_ERR_CUDA, "preprocess horizontal pass: %s", cudaGetErrorString(e));
     // vertical pass (identity table when oh == Hs: one tap of weight 1 << 22 -> exact copy)
@@ -1648,14 +1688,14 @@ static int preprocess_impl(fvhd_handle h, cudaStream_t st, const void* rgb, int 
     const int* yb = (const int*)ty.bounds; const int* yk = (const int*)ty.kk; const float* lut = (const float*)h->rs_lut; const uint8_t* tmp = (const uint8_t*)h->rs_tmp;
     if (tiles_y * tiles_x == 1 && top >= 0 && left >= 0 && top + R <= oh && left + R <= ow) {       // one window inside the image
         const dim3 g2((R + 127) / 128, R);
-        if (out_dtype == FVHD_F32) e = launch_k(resample_v_crop_kernel<float>, g2, dim3(128), 0, st, tmp, ow, (float*)out, R, top, left, yb, yk, ty.ksize, lut);
-        else if (out_dtype == FVHD_F16) e = launch_k(resample_v_crop_kernel<__half>, g2, dim3(128), 0, st, tmp, ow, (__half*)out, R, top, left, yb, yk, ty.ksize, lut);
-        else e = launch_k(resample_v_crop_kernel<bf16>, g2, dim3(128), 0, st, tmp, ow, (bf16*)out, R, top, left, yb, yk, ty.ksize, lut);
+        if (out_dtype == FVHD_F32) e = launch_k(pdl, resample_v_crop_kernel<float>, g2, dim3(128), 0, st, tmp, ow, (float*)out, R, top, left, yb, yk, ty.ksize, lut);
+        else if (out_dtype == FVHD_F16) e = launch_k(pdl, resample_v_crop_kernel<__half>, g2, dim3(128), 0, st, tmp, ow, (__half*)out, R, top, left, yb, yk, ty.ksize, lut);
+        else e = launch_k(pdl, resample_v_crop_kernel<bf16>, g2, dim3(128), 0, st, tmp, ow, (bf16*)out, R, top, left, yb, yk, ty.ksize, lut);
     } else {                                                                                         // tiles of a canvas: black outside the image
         const dim3 g2((R + 127) / 128, R, tiles_y * tiles_x);
-        if (out_dtype == FVHD_F32) e = launch_k(resample_v_tiles_kernel<float>, g2, dim3(128), 0, st, tmp, ow, oh, (float*)out, R, top, left, tiles_x, yb, yk, ty.ksize, lut);
-        else if (out_dtype == FVHD_F16) e = launch_k(resample_v_tiles_kernel<__half>, g2, dim3(128), 0, st, tmp, ow, oh, (__half*)out, R, top, left, tiles_x, yb, yk, ty.ksize, lut);
-        else e = launch_k(resample_v_tiles_kernel<bf16>, g2, dim3(128), 0, st, tmp, ow, oh, (bf16*)out, R, top, left, tiles_x, yb, yk, ty.ksize, lut);
+        if (out_dtype == FVHD_F32) e = launch_k(pdl, resample_v_tiles_kernel<float>, g2, dim3(128), 0, st, tmp, ow, oh, (float*)out, R, top, left, tiles_x, yb, yk, ty.ksize, lut);
+        else if (out_dtype == FVHD_F16) e = launch_k(pdl, resample_v_tiles_kernel<__half>, g2, dim3(128), 0, st, tmp, ow, oh, (__half*)out, R, top, left, tiles_x, yb, yk, ty.ksize, lut);
+        else e = launch_k(pdl, resample_v_tiles_kernel<bf16>, g2, dim3(128), 0, st, tmp, ow, oh, (bf16*)out, R, top, left, tiles_x, yb, yk, ty.ksize, lut);
     }
     if (e != cudaSuccess) return fail(h, FVHD_ERR_CUDA, "preprocess vertical pass: %s", cudaGetErrorString(e));
     return FVHD_OK;
@@ -1694,7 +1734,7 @@ int fvhd_preprocess_tiles(fvhd_handle h, void* stream, const void* rgb, int src_
 int fvhd_debug_gemm_trace(void* dev_buf_16_u64_per_cta, int force_bn, int max_cs) {
     g_gemm_trace = reinterpret_cast<unsigned long long*>(dev_buf_16_u64_per_cta);
     g_force_bn = force_bn;
-    if (max_cs == 1 || max_cs == 2 || max_cs == 4) g_gemm_max_cs = max_cs;
+    if (max_cs == 1 || max_cs == 2 || max_cs == 4) g_debug_gemm_cs = max_cs;
     return FVHD_OK;
 }
 
@@ -1710,10 +1750,7 @@ int fvhd_gemm(fvhd_handle h, void* stream, const void* A, const void* W, const v
     Step s;
     if ((rc = make_gemm_step(h, &s, nullptr, 1, (const bf16*)A, K, (const bf16*)W, (const float*)bias, (const bf16*)residual, N, (bf16*)D, N, M, N, K, act)) != FVHD_OK) return rc;
     if (!D) return fail(h, FVHD_ERR_INVALID, "D is null");
-    RunCtx ctx{};
-    cudaError_t e = s(reinterpret_cast<cudaStream_t>(stream), ctx);
-    if (e != cudaSuccess) return fail(h, FVHD_ERR_CUDA, "gemm launch failed: %s", cudaGetErrorString(e));
-    return FVHD_OK;
+    return launch_step(h, s, stream, "gemm");
 }
 
 int fvhd_convffn_half(fvhd_handle h, void* stream, const void* z, const void* w1, const void* b1, const void* w2, int w2_is_f16, const void* b2,
@@ -1725,10 +1762,7 @@ int fvhd_convffn_half(fvhd_handle h, void* stream, const void* z, const void* w1
     Step s;
     if ((rc = make_convffn2_step(h, &s, (const bf16*)z, (const bf16*)w1, (const float*)b1, w2, w2_is_f16, (const float*)b2,
                                  (const bf16*)resid, (bf16*)out, M, C)) != FVHD_OK) return rc;
-    RunCtx ctx{};
-    cudaError_t e = s(reinterpret_cast<cudaStream_t>(stream), ctx);
-    if (e != cudaSuccess) return fail(h, FVHD_ERR_CUDA, "convffn2 launch failed: %s", cudaGetErrorString(e));
-    return FVHD_OK;
+    return launch_step(h, s, stream, "convffn2");
 }
 
 int fvhd_attention(fvhd_handle h, void* stream, const void* qkv, void* out, int batch, int N, int C) {
@@ -1738,17 +1772,9 @@ int fvhd_attention(fvhd_handle h, void* stream, const void* qkv, void* out, int 
     if (!qkv || !out || batch < 1 || N < 1 || C < 32 || C % 32) return fail(h, FVHD_ERR_INVALID, "fvhd_attention: bad arguments");
     const float sl2 = 0.17677669529663687f * 1.4426950408889634f;
     Step s;
-    if (g_attn_mode == 'u') {
-        if ((rc = make_attention_umma_step(h, &s, (const bf16*)qkv, (bf16*)out, batch, N, C, sl2)) != FVHD_OK) return rc;
-    } else {
-        const dim3 agrid((N + 63) / 64, C / 32, batch);
-        const bf16* q_ = (const bf16*)qkv; bf16* o_ = (bf16*)out;
-        s = [=](cudaStream_t st, const RunCtx&) -> cudaError_t { return launch_k(attention_kernel, agrid, dim3(128), 0, st, q_, o_, N, C, sl2); };
-    }
-    RunCtx ctx{};
-    cudaError_t e = s(reinterpret_cast<cudaStream_t>(stream), ctx);
-    if (e != cudaSuccess) return fail(h, FVHD_ERR_CUDA, "attention launch failed: %s", cudaGetErrorString(e));
-    return FVHD_OK;
+    if ((rc = (h->opt.attn == 'u' ? make_attention_umma_step : make_attention_mma_step)(h, &s, (const bf16*)qkv, (bf16*)out, batch, N, C, sl2)) != FVHD_OK)
+        return rc;
+    return launch_step(h, s, stream, "attention");
 }
 
 int fvhd_mixer(fvhd_handle h, void* stream, const void* x, const void* w3, const void* b3, const void* w7, const void* b7,
@@ -1757,41 +1783,12 @@ int fvhd_mixer(fvhd_handle h, void* stream, const void* x, const void* w3, const
     int rc = ensure_cuda(h);
     if (rc != FVHD_OK) return rc;
     if (!x || !w3 || !b3 || !w7 || !b7 || !y || !z || batch < 1 || H < 1 || W < 1) return fail(h, FVHD_ERR_INVALID, "fvhd_mixer: null operand or empty shape");
+    const char m = h->opt.mixer;
+    const Mixer k = m == '2' ? Mixer::Tc2 : m == 't' ? Mixer::Tc : (m == 0 || m == 'z') ? Mixer::Tz : Mixer::Umma;
     Step s;
-    if (g_mixer_mode == '2') {      // FVHD_MIXER=2: the mma.sync kernel of mixer_tc2.cuh; otherwise the tcgen05 diagonal-tap kernel
-        if (C % MixT2::CG) return fail(h, FVHD_ERR_INVALID, "fvhd_mixer: C %% 16 != 0");
-        const int tx2 = (W + MixT2::TOW - 1) / MixT2::TOW, ty2 = (H + MixT2::TOH - 1) / MixT2::TOH;
-        const dim3 grid2(tx2 * ty2, C / MixT2::CG, batch);
-        CUtensorMap tm2;
-        if ((rc = make_tmap_nhwc(h, &tm2, x, batch, H, W, C, MixT2::XP, MixT2::XH, MixT2::CG)) != FVHD_OK) return rc;
-        bf16 *y2 = (bf16*)y, *z2 = (bf16*)z;
-        const float *w3f = (const float*)w3, *b3f = (const float*)b3, *w7f = (const float*)w7, *b7f = (const float*)b7;
-        s = [=](cudaStream_t st, const RunCtx&) -> cudaError_t {
-            return launch_k(repmixer_tc2_kernel, grid2, dim3(MixT2::NT), MixT2::SMEM, st, tm2, y2, z2, w3f, b3f, w7f, b7f, H, W, C, tx2);
-        };
-    } else if (g_mixer_mode == 't') {   // FVHD_MIXER=t: the mma.sync-7x7 kernel of mixer_tc.cuh (32-channel groups)
-        if (C % DW_CG) return fail(h, FVHD_ERR_INVALID, "fvhd_mixer: C %% 32 != 0");
-        const int tx = (W + 15) / 16, ty = (H + 15) / 16;
-        int per_group = (2 * h->num_sms) / (C / DW_CG);
-        if (per_group < 1) per_group = 1;
-        if (per_group > tx * ty * batch) per_group = tx * ty * batch;
-        const dim3 grid_tc(per_group, C / DW_CG, 1);
-        CUtensorMap tmx;
-        if ((rc = make_tmap_nhwc(h, &tmx, x, batch, H, W, C, MixTc::XP, MixTc::XH)) != FVHD_OK) return rc;
-        bf16 *y2 = (bf16*)y, *z2 = (bf16*)z;
-        const float *w3f = (const float*)w3, *b3f = (const float*)b3, *w7f = (const float*)w7, *b7f = (const float*)b7;
-        s = [=](cudaStream_t st, const RunCtx&) -> cudaError_t {
-            return launch_k(repmixer_tc_kernel, grid_tc, dim3(MixTc::NT), MixTc::SMEM, st, tmx, y2, z2, w3f, b3f, w7f, b7f, H, W, C, tx, batch);
-        };
-    } else if (g_mixer_mode == 'z') {   // FVHD_MIXER=z: Toeplitz tcgen05 kernel (mixer_tz.cuh)
-        if ((rc = make_mixer_tz_step(h, &s, (const bf16*)x, (bf16*)y, (bf16*)z, (const float*)w3, (const float*)b3, (const float*)w7,
-                                     (const float*)b7, batch, H, W, C)) != FVHD_OK) return rc;
-    } else if ((rc = make_mixer_umma_step(h, &s, (const bf16*)x, (bf16*)y, (bf16*)z, (const float*)w3, (const float*)b3, (const float*)w7,
+    if ((rc = kMixers[(int)k].make(h, &s, (const bf16*)x, (bf16*)y, (bf16*)z, (const float*)w3, (const float*)b3, (const float*)w7,
                                    (const float*)b7, batch, H, W, C)) != FVHD_OK) return rc;
-    RunCtx ctx{};
-    cudaError_t e = s(reinterpret_cast<cudaStream_t>(stream), ctx);
-    if (e != cudaSuccess) return fail(h, FVHD_ERR_CUDA, "mixer launch failed: %s", cudaGetErrorString(e));
-    return FVHD_OK;
+    return launch_step(h, s, stream, "mixer");
 }
 
 int fvhd_convffn(fvhd_handle h, void* stream, const void* z, const void* w1, const void* b1, const void* w2, const void* b2,
@@ -1811,10 +1808,7 @@ int fvhd_convffn(fvhd_handle h, void* stream, const void* z, const void* w1, con
         return fail(h, FVHD_ERR_INVALID, "fvhd_convffn: fused ConvFFN kernels exist for C in {96, 192, 384}, got %d", C);
     }
     if (rc != FVHD_OK) return rc;
-    RunCtx ctx{};
-    cudaError_t e = s(reinterpret_cast<cudaStream_t>(stream), ctx);
-    if (e != cudaSuccess) return fail(h, FVHD_ERR_CUDA, "convffn launch failed: %s", cudaGetErrorString(e));
-    return FVHD_OK;
+    return launch_step(h, s, stream, "convffn");
 }
 
 

@@ -278,7 +278,7 @@ class Engine:
         return out
 
     def attention(self, qkv, batch, n_tokens):
-        """MHSA core on qkv [B*N, 3C] bf16 -> [B*N, C] bf16 (kernel per FVHD_ATTN at handle creation)."""
+        """MHSA core on qkv [B*N, 3C] bf16 -> [B*N, C] bf16 (kernel per FVHD_ATTN as it was when the engine was created)."""
         Cc = qkv.shape[1] // 3
         out = torch.empty(qkv.shape[0], Cc, dtype=torch.bfloat16, device=qkv.device)
         with torch.cuda.device(qkv.device):
@@ -287,7 +287,8 @@ class Engine:
         return out
 
     def mixer(self, x, w3, b3, w7, b7):
-        """(y, z) = (dw3x3(x) + b3, dw7x7(y) + b7) on the tcgen05 mixer kernel; x bf16 NHWC [B,H,W,C], weights fp32 tap-major."""
+        """(y, z) = (dw3x3(x) + b3, dw7x7(y) + b7) on the mixer kernel FVHD_MIXER selected when the engine was created; x bf16 NHWC
+        [B,H,W,C], weights fp32 tap-major."""
         B, H, W, Cc = x.shape
         y = torch.empty_like(x)
         z = torch.empty_like(x)

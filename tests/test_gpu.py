@@ -150,14 +150,15 @@ def test_every_unit_isolated_256(eng256, oracle256, dev):
     assert not bad, bad
 
 
-def _engine_with_env(R, packed, dev, env):
-    """Engine whose batch-1 plan is built under the given environment switches (read when a handle first touches CUDA / builds a plan)."""
-    keys = ("FVHD_MIX_TILE", "FVHD_MIXER")
+def _engine_with_env(R, packed, dev, env, batch=1):
+    """Engine created, and its first plan built, under the given environment switches (the library reads them once per handle,
+    when the handle is created); the mixer / ConvFFN switches the caller does not name are unset meanwhile."""
+    keys = {"FVHD_MIX_TILE", "FVHD_MIXER", "FVHD_NO_FUSED_MLP", "FVHD_NO_CLUSTER_MLP", "FVHD_CONVFFN", *env}
     old = {k: os.environ.pop(k, None) for k in keys}
     os.environ.update(env)
     try:
-        eng = pkg.Engine(R, 896, 2, 1).load(packed, dev)
-        eng.forward(fx.synthetic_images(1, R).to(dev), False, True)
+        eng = pkg.Engine(R, 896, 2, batch).load(packed, dev)
+        eng.forward(fx.synthetic_images(batch, R).to(dev), False, True)
     finally:
         for k in keys:
             os.environ.pop(k, None)
@@ -292,22 +293,15 @@ def test_missing_weights_and_workspace_fail_loudly(packed, dev):
 
 def test_fused_convffn_is_bit_identical_to_two_gemms(packed, dev):
     """mlp_fused_tcgen05_kernel keeps the fc2 accumulation order of the unfused path (hidden chunk j == k-block j), so the
-    whole forward must agree BIT FOR BIT with FVHD_NO_FUSED_MLP=1 (evaluated in a subprocess: the switch is read once)."""
-    import subprocess, sys, tempfile
-    code = (
-        "import sys, torch; sys.path.insert(0, %r)\n"
-        "import ml_fastvlm_b200 as pkg; from oracle import fixture as fx\n"
-        "pk = pkg.pack_tower(fx.tower_state_dict()); pk.update(pkg.pack_projector(fx.projector_state_dict(896)))\n"
-        "eng = pkg.Engine(512, 896, 2, 2).load(pk, torch.device('cuda:0'))\n"
-        "t, p = eng.forward(fx.synthetic_images(2, 512, seed=4).to('cuda:0'), True, True)\n"
-        "torch.save({'t': t.cpu(), 'p': p.cpu(), 'launches': eng.launches_per_forward(2)}, sys.argv[1])\n" % os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
-    outs = []
-    for env_val in ("0", "1"):
-        f = tempfile.NamedTemporaryFile(suffix=".pt", delete=False).name
-        env = dict(os.environ, FVHD_NO_FUSED_MLP=env_val, FVHD_NO_CLUSTER_MLP="1", FVHD_CONVFFN="1")     # first-generation fused kernel
-        subprocess.run([sys.executable, "-c", code, f], check=True, env=env, timeout=300)
-        outs.append(torch.load(f))
-        os.unlink(f)
+    whole forward must agree BIT FOR BIT with FVHD_NO_FUSED_MLP=1 (each variant on its own engine, created under its switches)."""
+    x = fx.synthetic_images(2, 512, seed=4).to(dev)
+
+    def run(env):
+        eng = _engine_with_env(512, packed, dev, env, batch=2)
+        t, p = eng.forward(x, True, True)
+        return {"t": t.cpu(), "p": p.cpu(), "launches": eng.launches_per_forward(2)}
+
+    outs = [run({"FVHD_NO_FUSED_MLP": v, "FVHD_NO_CLUSTER_MLP": "1", "FVHD_CONVFFN": "1"}) for v in ("0", "1")]     # first-generation fused kernel
     assert outs[0]["launches"] == outs[1]["launches"] - 14            # 2 + 12 RepMixer blocks lose one launch each
     assert torch.isfinite(outs[0]["p"].float()).all()
     assert torch.equal(outs[0]["t"], outs[1]["t"]) and torch.equal(outs[0]["p"], outs[1]["p"])
@@ -316,21 +310,14 @@ def test_fused_convffn_is_bit_identical_to_two_gemms(packed, dev):
     # per block, which this random-weight fixture amplifies ~70x through the remaining depth (tests/golden/sensitivity.json;
     # the reference's own bf16 run sits 3.8e-2 from its fp32 run).  Bound: two valid bf16 pipelines must agree to that
     # level; parity of the cluster path itself is checked unit by unit and end to end against the oracle above.
-    f = tempfile.NamedTemporaryFile(suffix=".pt", delete=False).name
-    subprocess.run([sys.executable, "-c", code, f], check=True, env=dict(os.environ, FVHD_NO_FUSED_MLP="0", FVHD_NO_CLUSTER_MLP="0", FVHD_CONVFFN="1"), timeout=300)
-    clus = torch.load(f)
-    os.unlink(f)
+    clus = run({"FVHD_NO_FUSED_MLP": "0", "FVHD_NO_CLUSTER_MLP": "0", "FVHD_CONVFFN": "1"})
     assert clus["launches"] == outs[0]["launches"] - 24               # 24 stage-2 blocks lose one launch each
     assert torch.isfinite(clus["p"].float()).all()
     dt, dp = rel_l2(clus["t"], outs[0]["t"]), rel_l2(clus["p"], outs[0]["p"])
     assert dt < 4e-2 and dp < 4e-2, (dt, dp)
     # the default plan (second-generation fused kernel, f16 hidden + packed-half GELU, convffn.cuh): same launch count as the
     # fully fused first-generation plan, and -- a different but equally valid rounding of the hidden -- within the same bound
-    f = tempfile.NamedTemporaryFile(suffix=".pt", delete=False).name
-    env = {k: v for k, v in os.environ.items() if k not in ("FVHD_CONVFFN", "FVHD_NO_FUSED_MLP", "FVHD_NO_CLUSTER_MLP")}
-    subprocess.run([sys.executable, "-c", code, f], check=True, env=env, timeout=300)
-    gen2 = torch.load(f)
-    os.unlink(f)
+    gen2 = run({})
     assert gen2["launches"] == clus["launches"]
     dt, dp = rel_l2(gen2["t"], outs[1]["t"]), rel_l2(gen2["p"], outs[1]["p"])
     assert torch.isfinite(gen2["p"].float()).all() and dt < 4e-2 and dp < 4e-2, (dt, dp)

@@ -239,10 +239,9 @@ def _mixer_ref(x_nhwc, w3, b3, w7, b7, round_weights):
 def test_umma_mixer_vs_torch(dev, B, H, W, C, mode):
     """mode z: Toeplitz tcgen05 kernel (mixer_tz.cuh, bf16 planes and taps); mode u: tcgen05 diagonal-tap kernel (mixer_umma.cuh, bf16
     taps); mode 2: both convs on mma.sync (mixer_tc2.cuh, f16 taps)."""
-    os.environ["FVHD_MIXER"] = mode                      # read when a handle first touches CUDA
+    os.environ["FVHD_MIXER"] = mode                      # read when the handle is created
     try:
         eng = pkg.Engine(64, 0, 2, 1)
-        eng.gemm(torch.zeros(8, 64, dtype=torch.bfloat16, device=dev), torch.zeros(8, 64, dtype=torch.bfloat16, device=dev))
     finally:
         os.environ.pop("FVHD_MIXER", None)
     g = torch.Generator().manual_seed(B * 1000 + H * 10 + C)
@@ -270,7 +269,6 @@ def test_umma_mixer_identity_taps(dev, mode):
     os.environ["FVHD_MIXER"] = mode
     try:
         eng = pkg.Engine(64, 0, 2, 1)
-        eng.gemm(torch.zeros(8, 64, dtype=torch.bfloat16, device=dev), torch.zeros(8, 64, dtype=torch.bfloat16, device=dev))
     finally:
         os.environ.pop("FVHD_MIXER", None)
     g = torch.Generator().manual_seed(1)
@@ -359,7 +357,6 @@ def test_attention_core_vs_torch(dev, B, N, C, mode):
     os.environ["FVHD_ATTN"] = mode
     try:
         eng = pkg.Engine(64, 0, 2, 1)
-        eng.gemm(torch.zeros(8, 64, dtype=torch.bfloat16, device=dev), torch.zeros(8, 64, dtype=torch.bfloat16, device=dev))
     finally:
         os.environ.pop("FVHD_ATTN", None)
     g = torch.Generator().manual_seed(N + C + B)
@@ -438,13 +435,14 @@ def test_repmixer_block_large_activations(packed, tower_sd, dev):
 
 
 # ------------------------------------------------------------------ plan variants: Toeplitz tcgen05 mixer, stem generations
-def _engine_env(R, packed, dev, env, batch=1):
-    """Engine whose plan is built under the given FVHD_* switches (read when a handle first touches CUDA / builds its plan)."""
-    keys = ("FVHD_MIX_TILE", "FVHD_MIXER", "FVHD_STEM")
+def _engine_env(R, packed, dev, env, batch=1, max_batch=None):
+    """Engine created, and its first plan (`batch` images) built, under the given FVHD_* switches (the library reads them once per
+    handle, when the handle is created); the mixer / stem switches the caller does not name are unset meanwhile."""
+    keys = {"FVHD_MIX_TILE", "FVHD_MIXER", "FVHD_STEM", *env}
     old = {k: os.environ.pop(k, None) for k in keys}
     os.environ.update(env)
     try:
-        eng = pkg.Engine(R, 896, 2, batch).load(packed, dev)
+        eng = pkg.Engine(R, 896, 2, max_batch or batch).load(packed, dev)
         eng.forward(fx.synthetic_images(batch, R).to(dev), False, True)
     finally:
         for k in keys:
@@ -514,7 +512,6 @@ def test_stem_generations_agree(packed, tower_sd, proj_sd, dev, R, B):
 def test_convffn2_weight_sharing_clusters_bit_identical(dev, C, M):
     """convffn_tcgen05_kernel<C, 2> (TMA-multicast weight ring shared by two CTAs; odd tile counts leave rank 1 one dummy tile) must
     reproduce the single-CTA kernel bit for bit: same MMAs in the same order, only the origin of the weight bytes differs."""
-    eng = pkg.Engine(64, 0, 2, 1)
     g = torch.Generator().manual_seed(3 * C + M)
     z = torch.randn(M, C, generator=g).to(torch.bfloat16).to(dev)
     w1 = (torch.randn(4 * C, C, generator=g) / C ** 0.5).to(torch.bfloat16).to(dev)
@@ -524,12 +521,13 @@ def test_convffn2_weight_sharing_clusters_bit_identical(dev, C, M):
     r = torch.randn(M, C, generator=g).to(torch.bfloat16).to(dev)
     outs = {}
     for cs in ("1", "2"):
-        os.environ["FVHD_CONVFFN_CS"] = cs
+        os.environ["FVHD_CONVFFN_CS"] = cs                # read when the handle is created: one engine per cluster size
         try:
-            outs[cs] = [eng.convffn2(z, w1, b1, w2h, b2, r) for _ in range(3)]
-            torch.cuda.synchronize()
+            eng = pkg.Engine(64, 0, 2, 1)
         finally:
             os.environ.pop("FVHD_CONVFFN_CS", None)
+        outs[cs] = [eng.convffn2(z, w1, b1, w2h, b2, r) for _ in range(3)]
+        torch.cuda.synchronize()
     ref = r.float() + torch.nn.functional.gelu(z.float() @ w1.float().t() + b1) .to(torch.float16).float() @ w2h.float().t() + b2
     assert rel_l2(outs["1"][0].float(), ref) < 6e-3
     for o in outs["2"]:
@@ -544,6 +542,42 @@ def test_default_plan_picks_mixer_per_launch(packed, dev):
     k4 = [s["kernel"] for s in eng.steps(4)]
     assert k1.count("repmixer_tz_kernel") == 14 and k1.count("repmixer_tc_kernel") == 24, (k1.count("repmixer_tz_kernel"), k1.count("repmixer_tc_kernel"))
     assert k4.count("repmixer_tz_kernel") == 38 and "repmixer_tc_kernel" not in k4
+
+
+def test_handles_keep_their_own_switches(packed, dev):
+    """Kernel-selection switches are read once per handle, when it is created: a handle created later without them changes
+    neither the plans nor the single-kernel entries of an earlier one, and is not affected by it either."""
+    a = _engine_env(256, packed, dev, {"FVHD_MIXER": "u"}, batch=1, max_batch=2)
+    b = _engine_env(256, packed, dev, {})
+    assert "repmixer_umma_kernel" in {s["kernel"] for s in a.steps(2)}          # A's batch-2 plan is built after B exists
+    g = torch.Generator().manual_seed(6)
+    x = torch.randn(1, 32, 32, 96, generator=g).to(torch.bfloat16).to(dev)
+    w3, b3 = (torch.randn(9, 96, generator=g) / 3).to(dev), (torch.randn(96, generator=g) * 0.1).to(dev)
+    w7, b7 = (torch.randn(49, 96, generator=g) / 7).to(dev), (torch.randn(96, generator=g) * 0.1).to(dev)
+    os.environ["FVHD_MIXER"] = "u"
+    try:
+        fresh_u = pkg.Engine(64, 0, 2, 1)
+    finally:
+        os.environ.pop("FVHD_MIXER", None)
+    ya, za = a.mixer(x, w3, b3, w7, b7)
+    yu, zu = fresh_u.mixer(x, w3, b3, w7, b7)
+    assert torch.equal(ya, yu) and torch.equal(za, zu)
+    fresh = _engine_env(256, packed, dev, {})
+    assert b.steps(1) == fresh.steps(1)
+    assert "repmixer_umma_kernel" not in {s["kernel"] for s in b.steps(1)}
+
+
+@pytest.mark.parametrize("env", [{}, {"FVHD_CONVFFN": "1"}, {"FVHD_NO_FUSED_MLP": "1"}])
+@pytest.mark.parametrize("R", [256, 1024])
+def test_launches_per_forward_is_the_plan(packed, dev, R, env):
+    """fvhd_launches_per_forward == the plan's kernels + set_io_kernel for every batch up to max_batch (at 1024 px the stage-2
+    ConvFFN kernel depends on the batch), and the sum over the passes above it."""
+    mb = 4
+    eng = _engine_env(R, packed, dev, env, batch=1, max_batch=mb)
+    per_pass = {b: len(eng.steps(b)) + 1 for b in range(1, mb + 1)}
+    for b, n in per_pass.items():
+        assert eng.launches_per_forward(b) == n, (b, n)
+    assert eng.launches_per_forward(2 * mb + 3) == 2 * per_pass[mb] + per_pass[3]
 
 
 # ------------------------------------------------------------------ row f4 on the GPU: released-layout checkpoint -> drop-in modules

@@ -19,21 +19,21 @@ dev = torch.device("cuda:0")
 SHAPES = [(256, 256, 96, 2), (128, 128, 192, 12), (64, 64, 384, 24)]       # H, W, C, blocks per forward
 
 
-def engine(mode):
+def engine(mode, skip):
+    """Engine whose fvhd_mixer runs `mode` with the FVHD_TZ_SKIP mask `skip` (switches are read when a handle is created)."""
     os.environ["FVHD_MIXER"] = mode
+    os.environ["FVHD_TZ_SKIP"] = str(skip)
     try:
-        eng = pkg.Engine(64, 0, 2, 1)
-        eng.gemm(torch.zeros(8, 64, dtype=torch.bfloat16, device=dev), torch.zeros(8, 64, dtype=torch.bfloat16, device=dev))
+        return pkg.Engine(64, 0, 2, 1)
     finally:
         os.environ.pop("FVHD_MIXER", None)
-    return eng
+        os.environ.pop("FVHD_TZ_SKIP", None)
 
 
 flush = torch.empty(256 << 20, dtype=torch.uint8, device=dev)
 for mode in modes:
-    eng = engine(mode)
     for B, skip in [(b, k) for b in batches for k in skips]:
-        os.environ["FVHD_TZ_SKIP"] = str(skip)
+        eng = engine(mode, skip)
         tot_us = 0.0
         for (H, W, C, nblk) in SHAPES:
             g = torch.Generator().manual_seed(H + C + B)

@@ -19,13 +19,19 @@ def main():
     x = fx.synthetic_images(1, R).to(dev).to(torch.bfloat16)
     for _ in range(3):
         eng.forward(x, False, True)
+    # one more forward with tracing on, launched step by step: a second engine, created under FVHD_NO_GRAPH=1 (switches are read
+    # when a handle is created); the buffer keeps the stamps of the last mixer launch
+    os.environ["FVHD_NO_GRAPH"] = "1"
+    try:
+        direct = pkg.Engine(R, 896, 2, 1).load(pk, dev)
+    finally:
+        os.environ.pop("FVHD_NO_GRAPH", None)
+    direct.forward(x, False, True)
     n = 4096
     buf = torch.zeros(n * 8, dtype=torch.int64, device=dev)
     eng.lib.fvhd_debug_mixer_trace(buf.data_ptr())
     last = [i for i, s in enumerate(eng.steps(1)) if s["kernel"].startswith("repmixer")][-1]
-    # run through the stage-2 tail only once more with tracing on (graph replay keeps the stamps of the last mixer launch)
-    os.environ["FVHD_NO_GRAPH"] = "1"
-    eng.forward(x, False, True)
+    direct.forward(x, False, True)
     torch.cuda.synchronize()
     eng.lib.fvhd_debug_mixer_trace(None)
     t = buf.cpu().numpy().reshape(n, 8).astype(np.float64)

@@ -19,6 +19,7 @@ N = 8
 
 
 def engine(mode):
+    """Engine created under the switches `mode` names (they are read when a handle is created)."""
     opts = mode.split(":")
     os.environ["FVHD_MIXER"] = opts[0]
     os.environ.pop("FVHD_NO_PDL", None)
@@ -36,7 +37,6 @@ def engine(mode):
             os.environ["FVHD_TZ_SKIP"] = o[4:]
     try:
         eng = pkg.Engine(64, 0, 2, 1)
-        eng.gemm(torch.zeros(8, 64, dtype=torch.bfloat16, device=dev), torch.zeros(8, 64, dtype=torch.bfloat16, device=dev))
     finally:
         os.environ.pop("FVHD_MIXER", None)
     return eng
